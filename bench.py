@@ -2,6 +2,7 @@
 """Benchmark of the DiffuScene denoising hot path on B200 (contract: see the task statement / DESIGN.md 5).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--scaling weak|strong]
+                    [--dump-outputs DIR]
 
 One "step" = one full T-step ancestral DDPM sample of the per-GPU batch: T denoiser forwards + T posterior updates,
 nothing skipped, per-step noise from the in-kernel Philox generator.  `value` = scenes/s with inputs resident in
@@ -55,6 +56,23 @@ CONFIGS = {
 }
 W_BYTES_BF16 = 155.35e6          # weights read once per step per GPU (SURVEY 8d)
 TEXT_L = 32
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: write each tensor as <out_dir>/<name>.npy (float64 stays float64, anything else becomes
+    float32) so that two builds can be compared output for output.  When the arrays come to more than DUMP_MAX_BYTES
+    in all, each keeps a fixed, seeded sample of rows along its first (scene) axis, in ascending order: the same rows
+    on every run with the same arguments."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: (v if v.dtype == torch.float64 else v.float()).detach().cpu() for k, v in arrays.items()}
+    total = sum(a.numel() * a.element_size() for a in arrays.values())
+    for name, a in arrays.items():
+        if total > DUMP_MAX_BYTES and a.dim() > 0:
+            keep = max(1, a.shape[0] * DUMP_MAX_BYTES // total)
+            a = a[torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
 
 
 def measured_peaks():
@@ -292,7 +310,14 @@ def main():
     ap.add_argument("--profile-ops", action="store_true", help="print the per-op device time table to stderr")
     ap.add_argument("--kv-hoist", type=int, default=1, help="text config: 1 = K/V of the text prefix precomputed once "
                     "per scene (default); 0 = recomputed before every diffusion step (what the reference does)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy: the sampled x_0 "
+                         "[scenes, N, d] (--config train: the loss)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.shape:
         args.config = {"real62": "bed_d62", "synth97": "bed_d97"}[args.shape]
     if args.config == "train":
@@ -374,9 +399,16 @@ def main():
 
     clocks = ClockSampler(local)
     clocks.start()
-    ms, launches, out = timed(resident_step, args.steps, args.warmup)
-    clk = clocks.stop()
+    try:
+        ms, launches, out = timed(resident_step, args.steps, args.warmup)
+    finally:                        # the sampler is a child process: never leave it polling after a failed step
+        clk = clocks.stop()
     assert torch.isfinite(out).all()
+    if args.dump_outputs:
+        from diffuscene_b200.parallel import gather_scenes
+        x0 = gather_scenes(out, B * world)          # a collective: every rank takes part
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"x0": x0})
     n_e2e = max(1, min(args.steps, 2))
     ms_e2e = None
     if not args.no_e2e:

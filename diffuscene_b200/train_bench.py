@@ -11,6 +11,7 @@ from __future__ import annotations
 import json
 import os
 import sys
+import tempfile
 import time
 
 import torch
@@ -20,11 +21,14 @@ F_TRAIN_MFLOP = 3 * 1455.7        # SURVEY 8d: training ~ 3 x forward FLOPs per 
 GLOBAL_BATCH = 8192
 
 
-def _config(tmp_stats):
+def _config():
+    """The training config; its `train_stats_file` is a private temporary file (a fixed name under a shared /tmp may
+    belong to another user), read once when the network is built: remove it after build_network()."""
     import yaml
     cfg = yaml.safe_load(open(os.path.join(ROOT, "config", "uncond/diffusion_livingrooms_instancond_lat32_v.yaml")).read().replace("\r", ""))
     from tests.cases import STATS
-    with open(tmp_stats, "w") as f:
+    fd, tmp_stats = tempfile.mkstemp(prefix="ds_b200_train_stats_", suffix=".json")
+    with os.fdopen(fd, "w") as f:
         json.dump(STATS, f)
     cfg["network"]["diffusion_kwargs"]["train_stats_file"] = tmp_stats
     cfg["network"]["diffusion_kwargs"]["loss_iou"] = True
@@ -50,13 +54,14 @@ def run_reference_train(args):
     kind = "port"
     B, N = 128, 21
     gen = torch.Generator().manual_seed(0)
-    cfg = _config("/tmp/ds_b200_train_stats.json")
     if "scene_synthesis" not in sys.modules and build_ref.activate():
         import contextlib
         import io
         from scene_synthesis.networks import build_network, optimizer_factory       # the vendored reference
+        cfg = _config()
         with contextlib.redirect_stdout(io.StringIO()):
             net, train_on_batch, _ = build_network(0, 26, cfg, None, "cpu")
+        os.remove(cfg["network"]["diffusion_kwargs"]["train_stats_file"])
         opt = optimizer_factory(cfg["training"], net.parameters())
         kind = "reference"
         sp = _batch(B, N, 25, gen)
@@ -97,14 +102,15 @@ def run_train_bench(args):
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     sys.path.insert(0, ROOT)
-    from bench import ClockSampler, measured_peaks
+    from bench import ClockSampler, dump_outputs, measured_peaks
     from scene_synthesis.networks import build_network, optimizer_factory
-    cfg = _config("/tmp/ds_b200_train_stats_%d.json" % rank)
+    cfg = _config()
     prec = args.precision or "bf16"
     B = args.batch or (GLOBAL_BATCH // world if args.scaling == "strong" else 1024)
     N = 21
     torch.manual_seed(0)
     net, train_on_batch, _ = build_network(0, 26, cfg, None, device=dev, precision=prec)
+    os.remove(cfg["network"]["diffusion_kwargs"]["train_stats_file"])
     opt = optimizer_factory(cfg["training"], net.parameters())
     gen = torch.Generator().manual_seed(1 + rank)
     host = {k: v.pin_memory() for k, v in _batch(B, N, 25, gen).items()}
@@ -141,8 +147,12 @@ def run_train_bench(args):
 
     clocks = ClockSampler(local)
     clocks.start()
-    ms, launches, last = timed(step_resident, args.steps, args.warmup)
-    clk = clocks.stop()
+    try:
+        ms, launches, last = timed(step_resident, args.steps, args.warmup)
+    finally:                        # the sampler is a child process: never leave it polling after a failed step
+        clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": torch.tensor([last], dtype=torch.float64)})
     phases = net.engine(commit=False).train_phase_ms()
     n_e2e = max(1, min(args.steps, 3))
     ms_e2e, _, _ = timed(step_e2e, n_e2e, 1)

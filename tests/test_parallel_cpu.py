@@ -1,5 +1,6 @@
 """CPU, world_size 2 over gloo: the scene-sharding host logic used by bench.py / multi-GPU sampling."""
 import os
+import socket
 
 import torch
 import torch.distributed as dist
@@ -18,6 +19,31 @@ def test_shard_range_partitions_exactly():
             assert seen == list(range(total))
 
 
+def _run_two_ranks(target):
+    """Start `target(rank, 2, port, q)` in two spawned processes and return what each put on q.  The port is one the
+    OS just handed out, so that concurrent runs of the suite do not meet at the same rendezvous; a rank still alive
+    when the test ends (its peer failed) is terminated rather than left waiting for the rendezvous."""
+    with socket.socket() as s:
+        s.bind(("127.0.0.1", 0))
+        port = s.getsockname()[1]
+    ctx = mp.get_context("spawn")
+    q = ctx.Queue()
+    procs = [ctx.Process(target=target, args=(r, 2, port, q)) for r in range(2)]
+    try:
+        for p in procs:
+            p.start()
+        res = [q.get(timeout=120) for _ in procs]
+        for p in procs:
+            p.join(timeout=60)
+            assert p.exitcode == 0
+        return res
+    finally:
+        for p in procs:
+            if p.is_alive():
+                p.terminate()
+                p.join()
+
+
 def _worker(rank, world, port, q):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
     dist.init_process_group("gloo", rank=rank, world_size=world)
@@ -31,16 +57,7 @@ def _worker(rank, world, port, q):
 
 
 def test_two_rank_gather_and_timing_reduce():
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    port = 29571
-    procs = [ctx.Process(target=_worker, args=(r, 2, port, q)) for r in range(2)]
-    for p in procs:
-        p.start()
-    res = [q.get(timeout=120) for _ in procs]
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    res = _run_two_ranks(_worker)
     for rank, scenes, ms in res:
         assert scenes == [float(i) for i in range(7)]       # global scene order, every scene exactly once
         assert ms == 11.0                                    # max over ranks
@@ -67,15 +84,7 @@ def _dp_worker(rank, world, port, q):
 def test_two_rank_gradient_mean_equals_full_batch_gradient():
     """Data-parallel training (SURVEY 8e): the bucketed all-reduce mean of per-rank gradients on equal shards is
     the gradient of the full-batch mean loss."""
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    procs = [ctx.Process(target=_dp_worker, args=(r, 2, 29573, q)) for r in range(2)]
-    for p in procs:
-        p.start()
-    res = [q.get(timeout=120) for _ in procs]
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    res = _run_two_ranks(_dp_worker)
     model = _make_model()
     g = torch.Generator().manual_seed(11)
     x, y = torch.randn(8, 6, generator=g), torch.randn(8, 4, generator=g)
