@@ -480,11 +480,10 @@ void launch_gn_bwd(const T* c, int ldc, const T* dy, int ldy, T* dc, int lddc, T
                    int64_t dfilm_row_stride, int n_scenes, int n_obj, int C, int groups, cudaStream_t s) {
   const int64_t warps = (int64_t)n_scenes * groups;
   if (warps <= 0) return;
-  static const int use_reg = getenv("DS_GN_REG") ? atoi(getenv("DS_GN_REG")) : 1;
-  if (use_reg && groups == 8 && C == 512 && n_obj == 12)
+  if (groups == 8 && C == 512 && n_obj == 12)
     k_gn_bwd_reg<T, 12><<<cdiv64(warps, 8), 256, 0, s>>>(c, ldc, dy, ldy, dc, lddc, dres, ldr, res_accumulate, gamma, beta, film,
                                                          dgamma, dbeta, dfilm, dfilm_row_stride, n_scenes, C);
-  else if (use_reg && groups == 8 && C == 512 && n_obj == 21)
+  else if (groups == 8 && C == 512 && n_obj == 21)
     k_gn_bwd_reg<T, 21><<<cdiv64(warps, 8), 256, 0, s>>>(c, ldc, dy, ldy, dc, lddc, dres, ldr, res_accumulate, gamma, beta, film,
                                                          dgamma, dbeta, dfilm, dfilm_row_stride, n_scenes, C);
   else

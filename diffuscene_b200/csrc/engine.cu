@@ -173,9 +173,8 @@ static int gemm_variant(const ds_handle* h, const Op& o) {
   // row-major kernel would fall back to 128-wide tiles (N % 256 != 0: to_qkv); the MMA-bound shapes keep the
   // row-major kernel, whose 128 x 256 tiles feed the tensor pipe better than 128 x 192 (measured, profiles/)
   if (o.kind == OP_GEMM && h->gnt_plain && tc_gnt_plain_supported(h->cfg.num_objects, o.N)) {
-    static const int force_all = getenv("DS_GNT_PLAIN_ALL") ? atoi(getenv("DS_GNT_PLAIN_ALL")) : 0;
     const int K = o.in0.k + (o.in1.buf >= 0 ? o.in1.k : 0);
-    if (force_all || K <= 128 || o.N % 256 != 0) return 3;
+    if (K <= 128 || o.N % 256 != 0) return 3;
   }
   return 0;
 }
@@ -523,7 +522,6 @@ extern "C" int ds_create(const ds_config* cfg, ds_handle** out) {
   }
   // fuse_level 2: the fused conv + GroupNorm ops use the channels-on-lanes tcgen05 kernel where it applies
   h->gnt = h->use_tc && cfg->fuse_level >= 2 && tc_gnt_supported(cfg->num_objects, h->plan.C);
-  if (const char* e = getenv("DS_GNT")) h->gnt = h->gnt && atoi(e) != 0;
   h->gnt_plain = h->gnt && cfg->fuse_level >= 3;
   cudaError_t e = cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking);
   if (e != cudaSuccess) {

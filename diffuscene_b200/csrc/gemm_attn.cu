@@ -67,7 +67,6 @@ struct AtEpi {
   bf16* o; int ldo;                 // [M, 128]
   int M, kblocks;
   uint64_t desc_hi;
-  int uni_issue;           // see tc_common.cuh (DS_TC_UNI)
 };
 
 __device__ __forceinline__ float at_exp2(float x) {
@@ -265,59 +264,47 @@ k_ln_qkv_attn(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ 
   const int kblocks = epi.kblocks;
 
   if (warp == 0) {
-    // TMA producer.  UNI: the whole warp walks the loop, one elected lane issues (see tc_common.cuh)
-    auto producer = [&](auto uni_tag) {
-      constexpr bool UNI = decltype(uni_tag)::value;
-      if (!UNI && lane != 0) return;
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        const int m0 = tile * Cfg::ROWS;
-        for (int kb = 0; kb < kblocks; ++kb) {
-          mbar_wait(empty_bar(stage), phase ^ 1u, err_flag, 21);
-          mbar_expect_tx_r<UNI>(full_bar(stage), AT_STAGE_BYTES);
-          const uint32_t sa = base + stage * AT_STAGE_BYTES;
-          tma_load_2d_r<UNI>(sa, &tm_x, kb * BK, m0, full_bar(stage));
+    // TMA producer: the whole warp walks the loop, one elected lane issues (see tc_common.cuh)
+    int stage = 0;
+    uint32_t phase = 0;
+    for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
+      const int m0 = tile * Cfg::ROWS;
+      for (int kb = 0; kb < kblocks; ++kb) {
+        mbar_wait(empty_bar(stage), phase ^ 1u, err_flag, 21);
+        mbar_expect_tx_elect(full_bar(stage), AT_STAGE_BYTES);
+        const uint32_t sa = base + stage * AT_STAGE_BYTES;
+        tma_load_2d_elect(sa, &tm_x, kb * BK, m0, full_bar(stage));
 #pragma unroll
-          for (int r3 = 0; r3 < 3; ++r3)      // W' slab: three boxes of 128 rows -> [384 rows][128 B]
-            tma_load_2d_r<UNI>(sa + A_BYTES + r3 * 128 * BK * 2, &tm_w, kb * BK, r3 * 128, full_bar(stage));
-          if (++stage == AT_STAGES) { stage = 0; phase ^= 1u; }
-        }
+        for (int r3 = 0; r3 < 3; ++r3)      // W' slab: three boxes of 128 rows -> [384 rows][128 B]
+          tma_load_2d_elect(sa + A_BYTES + r3 * 128 * BK * 2, &tm_w, kb * BK, r3 * 128, full_bar(stage));
+        if (++stage == AT_STAGES) { stage = 0; phase ^= 1u; }
       }
-    };
-    if (epi.uni_issue) producer(std::true_type{});
-    else producer(std::false_type{});
+    }
   } else if (warp == 1) {
     // MMA issuer
-    auto issuer = [&](auto uni_tag) {
-      constexpr bool UNI = decltype(uni_tag)::value;
-      if (!UNI && lane != 0) return;
-      int stage = 0;
-      uint32_t phase = 0, tphase = 0;
-      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        mbar_wait(tempty_bar, tphase ^ 1u, err_flag, 22);
-        tphase ^= 1u;
+    int stage = 0;
+    uint32_t phase = 0, tphase = 0;
+    for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
+      mbar_wait(tempty_bar, tphase ^ 1u, err_flag, 22);
+      tphase ^= 1u;
+      tc_fence_after();
+      for (int kb = 0; kb < kblocks; ++kb) {
+        mbar_wait(full_bar(stage), phase, err_flag, 23);
         tc_fence_after();
-        for (int kb = 0; kb < kblocks; ++kb) {
-          mbar_wait(full_bar(stage), phase, err_flag, 23);
-          tc_fence_after();
-          const uint32_t sa = base + stage * AT_STAGE_BYTES;
-          const uint64_t adesc = umma_desc(sa, epi.desc_hi);
-          const uint64_t b0 = umma_desc(sa + A_BYTES, epi.desc_hi);
-          const uint64_t b1 = umma_desc(sa + A_BYTES + 256 * BK * 2, epi.desc_hi);
+        const uint32_t sa = base + stage * AT_STAGE_BYTES;
+        const uint64_t adesc = umma_desc(sa, epi.desc_hi);
+        const uint64_t b0 = umma_desc(sa + A_BYTES, epi.desc_hi);
+        const uint64_t b1 = umma_desc(sa + A_BYTES + 256 * BK * 2, epi.desc_hi);
 #pragma unroll
-          for (int k = 0; k < BK / 16; ++k) {
-            umma_issue<UNI>(tmem_base, adesc + uint64_t(2 * k), b0 + uint64_t(2 * k), AT_IDESC_256, (kb | k) != 0);
-            umma_issue<UNI>(tmem_base + 256u, adesc + uint64_t(2 * k), b1 + uint64_t(2 * k), AT_IDESC_128, (kb | k) != 0);
-          }
-          umma_arrive<UNI>(empty_bar(stage));
-          if (++stage == AT_STAGES) { stage = 0; phase ^= 1u; }
+        for (int k = 0; k < BK / 16; ++k) {
+          umma_issue_elect(tmem_base, adesc + uint64_t(2 * k), b0 + uint64_t(2 * k), AT_IDESC_256, (kb | k) != 0);
+          umma_issue_elect(tmem_base + 256u, adesc + uint64_t(2 * k), b1 + uint64_t(2 * k), AT_IDESC_128, (kb | k) != 0);
         }
-        umma_arrive<UNI>(tfull_bar);
+        umma_arrive_elect(empty_bar(stage));
+        if (++stage == AT_STAGES) { stage = 0; phase ^= 1u; }
       }
-    };
-    if (epi.uni_issue) issuer(std::true_type{});
-    else issuer(std::false_type{});
+      umma_arrive_elect(tfull_bar);
+    }
   } else {
     // ---------------- epilogue / core warps ----------------
     const int ew = warp - 2;                     // 0..15
@@ -471,7 +458,6 @@ AttnQkvPlan* attn_qkv_plan_create(const void* x, int ldx, const void* w, int ldw
   p->epi.ldo = ldo;
   p->epi.kblocks = K / BK;
   p->epi.desc_hi = umma_desc_hi_sw128();
-  p->epi.uni_issue = tc_uniform_issue();
   p->n_obj = n_obj;
   p->num_sms = tc_num_sms();
   return p;
@@ -486,7 +472,7 @@ int launch_ln_qkv_attn(const AttnQkvPlan* p, int M, cudaStream_t s) {
   const int tiles = (n_scenes + spt - 1) / spt;
   if (tiles == 0) return 0;
   const int grid = tiles < p->num_sms ? tiles : p->num_sms;
-  const bool pdl = tc_pdl_enabled(M);
+  const bool pdl = pdl_enabled(M);
   if (p->n_obj == 21)
     return tc_launch(k_ln_qkv_attn<21>, grid, AT_THREADS, AtCfg<21>::SMEM, s, pdl, p->tm_x, p->tm_w, epi, tc_error_flag_dev());
   return tc_launch(k_ln_qkv_attn<12>, grid, AT_THREADS, AtCfg<12>::SMEM, s, pdl, p->tm_x, p->tm_w, epi, tc_error_flag_dev());

@@ -55,7 +55,6 @@ struct LnEpi {
   const bf16* res; int ldres;      // residual added after the norm, or nullptr
   int M, kblocks;
   uint64_t desc_hi;
-  int uni_issue;           // see tc_common.cuh (DS_TC_UNI)
 };
 
 __global__ void __launch_bounds__(LN_THREADS, 1)
@@ -104,60 +103,48 @@ k_gemm_ln(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUte
   const int kblocks = epi.kblocks;
 
   if (warp == 0) {
-    // TMA producer.  UNI: the whole warp walks the loop, one elected lane issues (see tc_common.cuh)
-    auto producer = [&](auto uni_tag) {
-      constexpr bool UNI = decltype(uni_tag)::value;
-      if (!UNI && lane != 0) return;
-      // the whole weight matrix, once: per k-block two boxes of 256 rows x 64 columns -> [512 rows][128 B] slabs
-      mbar_expect_tx_r<UNI>(wfull_bar, uint32_t(kblocks * LN_C * BK * 2));
+    // TMA producer: the whole warp walks the loop, one elected lane issues (see tc_common.cuh)
+    // the whole weight matrix, once: per k-block two boxes of 256 rows x 64 columns -> [512 rows][128 B] slabs
+    mbar_expect_tx_elect(wfull_bar, uint32_t(kblocks * LN_C * BK * 2));
+    for (int kb = 0; kb < kblocks; ++kb) {
+      tma_load_2d_elect(base + uint32_t(kb * LN_C * BK * 2), &tm_w, kb * BK, 0, wfull_bar);
+      tma_load_2d_elect(base + uint32_t(kb * LN_C * BK * 2 + 256 * BK * 2), &tm_w, kb * BK, 256, wfull_bar);
+    }
+    int stage = 0;
+    uint32_t phase = 0;
+    for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
       for (int kb = 0; kb < kblocks; ++kb) {
-        tma_load_2d_r<UNI>(base + uint32_t(kb * LN_C * BK * 2), &tm_w, kb * BK, 0, wfull_bar);
-        tma_load_2d_r<UNI>(base + uint32_t(kb * LN_C * BK * 2 + 256 * BK * 2), &tm_w, kb * BK, 256, wfull_bar);
+        mbar_wait(empty_bar(stage), phase ^ 1u, err_flag, 11);
+        mbar_expect_tx_elect(full_bar(stage), A_BYTES);
+        tma_load_2d_elect(base + LN_A_OFF + stage * A_BYTES, &tm_a, kb * BK, tile * BM, full_bar(stage));
+        if (++stage == LN_STAGES) { stage = 0; phase ^= 1u; }
       }
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        for (int kb = 0; kb < kblocks; ++kb) {
-          mbar_wait(empty_bar(stage), phase ^ 1u, err_flag, 11);
-          mbar_expect_tx_r<UNI>(full_bar(stage), A_BYTES);
-          tma_load_2d_r<UNI>(base + LN_A_OFF + stage * A_BYTES, &tm_a, kb * BK, tile * BM, full_bar(stage));
-          if (++stage == LN_STAGES) { stage = 0; phase ^= 1u; }
-        }
-      }
-    };
-    if (epi.uni_issue) producer(std::true_type{});
-    else producer(std::false_type{});
+    }
   } else if (warp == 1) {
     // MMA issuer
-    auto issuer = [&](auto uni_tag) {
-      constexpr bool UNI = decltype(uni_tag)::value;
-      if (!UNI && lane != 0) return;
-      mbar_wait(wfull_bar, 0, err_flag, 12);
-      int stage = 0;
-      uint32_t phase = 0, tphase = 0;
-      for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        mbar_wait(tempty_bar, tphase ^ 1u, err_flag, 13);      // the epilogue has drained the accumulator
-        tphase ^= 1u;
+    mbar_wait(wfull_bar, 0, err_flag, 12);
+    int stage = 0;
+    uint32_t phase = 0, tphase = 0;
+    for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
+      mbar_wait(tempty_bar, tphase ^ 1u, err_flag, 13);      // the epilogue has drained the accumulator
+      tphase ^= 1u;
+      tc_fence_after();
+      for (int kb = 0; kb < kblocks; ++kb) {
+        mbar_wait(full_bar(stage), phase, err_flag, 14);
         tc_fence_after();
-        for (int kb = 0; kb < kblocks; ++kb) {
-          mbar_wait(full_bar(stage), phase, err_flag, 14);
-          tc_fence_after();
-          const uint64_t adesc = umma_desc(base + LN_A_OFF + stage * A_BYTES, epi.desc_hi);
-          const uint64_t b0 = umma_desc(base + uint32_t(kb * LN_C * BK * 2), epi.desc_hi);
-          const uint64_t b1 = umma_desc(base + uint32_t(kb * LN_C * BK * 2 + 256 * BK * 2), epi.desc_hi);
+        const uint64_t adesc = umma_desc(base + LN_A_OFF + stage * A_BYTES, epi.desc_hi);
+        const uint64_t b0 = umma_desc(base + uint32_t(kb * LN_C * BK * 2), epi.desc_hi);
+        const uint64_t b1 = umma_desc(base + uint32_t(kb * LN_C * BK * 2 + 256 * BK * 2), epi.desc_hi);
 #pragma unroll
-          for (int k = 0; k < BK / 16; ++k) {
-            umma_issue<UNI>(tmem_base, adesc + uint64_t(2 * k), b0 + uint64_t(2 * k), LN_IDESC, (kb | k) != 0);
-            umma_issue<UNI>(tmem_base + 256u, adesc + uint64_t(2 * k), b1 + uint64_t(2 * k), LN_IDESC, (kb | k) != 0);
-          }
-          umma_arrive<UNI>(empty_bar(stage));
-          if (++stage == LN_STAGES) { stage = 0; phase ^= 1u; }
+        for (int k = 0; k < BK / 16; ++k) {
+          umma_issue_elect(tmem_base, adesc + uint64_t(2 * k), b0 + uint64_t(2 * k), LN_IDESC, (kb | k) != 0);
+          umma_issue_elect(tmem_base + 256u, adesc + uint64_t(2 * k), b1 + uint64_t(2 * k), LN_IDESC, (kb | k) != 0);
         }
-        umma_arrive<UNI>(tfull_bar);
+        umma_arrive_elect(empty_bar(stage));
+        if (++stage == LN_STAGES) { stage = 0; phase ^= 1u; }
       }
-    };
-    if (epi.uni_issue) issuer(std::true_type{});
-    else issuer(std::false_type{});
+      umma_arrive_elect(tfull_bar);
+    }
   } else {
     // ---------------- epilogue warps ----------------
     const int q = warp & 3;                        // TMEM lane quadrant
@@ -382,7 +369,6 @@ LnGemmPlan* ln_plan_create(const GemmArgs& g, int rows_capacity, char* err, int 
   p->epi.M = g.M;
   p->epi.kblocks = g.k0 / BK;
   p->epi.desc_hi = umma_desc_hi_sw128();
-  p->epi.uni_issue = tc_uniform_issue();
   p->num_sms = tc_num_sms();
   return p;
 }
@@ -394,7 +380,7 @@ int launch_gemm_ln(const LnGemmPlan* p, int M, cudaStream_t s) {
   const int tiles = (M + BM - 1) / BM;
   if (tiles == 0) return 0;
   const int grid = tiles < p->num_sms ? tiles : p->num_sms;
-  return tc_launch(k_gemm_ln, grid, LN_THREADS, LN_SMEM, s, tc_pdl_enabled(M), p->tm_a, p->tm_w, epi, tc_error_flag_dev());
+  return tc_launch(k_gemm_ln, grid, LN_THREADS, LN_SMEM, s, pdl_enabled(M), p->tm_a, p->tm_w, epi, tc_error_flag_dev());
 }
 
 }  // namespace ds

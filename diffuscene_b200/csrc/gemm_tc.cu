@@ -65,11 +65,6 @@ struct TcEpi {
   int plain;             // channels-on-lanes kernel without GroupNorm: bias, activation, residual only
   float* d32;            // row-major plain kernel: fp32 output accumulated with atomics (split-K weight-gradient GEMMs)
   int ksplit;            // ... number of K splits (work units = tiles x ksplit)
-  int wide_pass1;        // channels-on-lanes kernel, N = 12: statistics pass reads its 48 TMEM columns with x32 + x16 loads
-  int two_cta;           // channels-on-lanes kernel, cluster of 2: cta_group::2 MMAs (bit 0 on, bit 2 shallow operand ring) (DS_GNT_2CTA)
-  int l2_prefetch;       // producers L2-prefetch the activation tile of their next work unit (A/B switch DS_TC_L2PF)
-  int uni_issue;         // producer / MMA warps run their loops warp-uniformly and elect the issuing lane (DS_TC_UNI)
-  int res_prefetch;      // channels-on-lanes kernel: L2-prefetch the next tile's residual rows (A/B switch DS_GNT_PREFETCH)
   unsigned long long* trace;   // optional [grid][8] cycle counters (bring-up / profiling aid), else nullptr
 };
 // trace slots: 0 producer wait-empty, 1 producer total, 2 mma wait-tmem-empty, 3 mma wait-full, 4 mma total,
@@ -149,11 +144,9 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant__ CUt
   // programmatic dependent launch: let the next kernel's CTAs be scheduled as SMs drain (its prologue overlaps
   // our tail); our own dependent work starts only after griddepcontrol.wait below
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  // thread-block cluster: the CS CTAs of a cluster work on CS consecutive M tiles of the same N tile and share
-  // the weight tile -- each CTA loads 1/CS of it and multicasts the slice into every CTA's shared memory
+  // cluster: 1 CTA, or the CTA pair (TWO), whose CTAs work on the 2 consecutive M tiles of the same N tile
   const uint32_t cs = cluster_nctarank();
   const uint32_t crank = cluster_ctarank();
-  const uint16_t cmask = uint16_t((1u << cs) - 1u);
 
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tm_a0);
@@ -163,7 +156,7 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant__ CUt
     // epilogue warps arrive on its tempty), empty[] / tfull[] get one arrival each from the leader's multicast commits
     for (int s = 0; s < Cfg::MAX_STAGES; ++s) {
       mbar_init(full_bar(s), 1);
-      mbar_init(empty_bar(s), TWO ? 1 : cs);       // multicast mode: every CTA of the cluster must have consumed the slot
+      mbar_init(empty_bar(s), 1);
     }
     for (int b = 0; b < 2; ++b) {
       mbar_init(tfull_bar(b), 1);
@@ -206,61 +199,40 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant__ CUt
   const int kb_per = (kblocks + ksplit - 1) / ksplit;
 
   if (warp == 0) {
-    // TMA producer.  UNI: the whole warp walks the loop, one elected lane issues (see tc_common.cuh)
-    auto producer = [&](auto uni_tag) {
-      constexpr bool UNI = decltype(uni_tag)::value;
-      if (!UNI && lane != 0) return;
-      int stage = 0;
-      uint32_t phase = 0;
-      unsigned long long tw = 0, tstart = clock64();
-      for (int unit = cluster_id; unit < total; unit += num_clusters) {
-        const int tile = unit % tiles_mn, kb_lo = (unit / tiles_mn) * kb_per, kb_hi = min(kblocks, kb_lo + kb_per);
-        const int n_idx = tile % num_n, m_idx = (tile / num_n) * int(cs) + int(crank);   // N fastest: neighbours share A in L2
-        const int m0 = m_idx * epi.tile_rows;
-        for (int kb = kb_lo; kb < kb_hi; ++kb) {
-          unsigned long long t0 = epi.trace ? clock64() : 0;
-          mbar_wait(empty_bar(stage), phase ^ 1u, err_flag, 1);
-          if (epi.trace) tw += clock64() - t0;
-          const uint32_t sa = base + stage * stb;
-          if constexpr (UNI && TWO) {      // CTA pair: own token tile + own half of the weight tile, bytes counted on the leader
-            if (crank == 0) mbar_expect_tx_r<true>(full_bar(stage), Cfg::STAGE_TX_2SM);
-            if (kb < epi.kb0) tma_load_2d_2sm_elect(sa, &tm_a0, kb * BK, m0, full_bar(stage));
-            else tma_load_2d_2sm_elect(sa, &tm_a1, (kb - epi.kb0) * BK, m0, full_bar(stage));
-            tma_load_2d_2sm_elect(sa + A_BYTES, &tm_w, kb * BK, n_idx * BN + int(crank) * (BN / 2), full_bar(stage));
-            if (++stage == nst) { stage = 0; phase ^= 1u; }
-            continue;
-          }
-          mbar_expect_tx_r<UNI>(full_bar(stage), Cfg::STAGE_BYTES);
-          if (kb < epi.kb0) tma_load_2d_r<UNI>(sa, &tm_a0, kb * BK, m0, full_bar(stage));
-          else tma_load_2d_r<UNI>(sa, &tm_a1, (kb - epi.kb0) * BK, m0, full_bar(stage));
-          if (epi.l2_prefetch && cs == 1 && n_idx == 0 && unit + num_clusters < tiles_mn) {      // see k_gemm_gnt
-            const int m1 = ((unit + num_clusters) / num_n) * epi.tile_rows;
-            if (kb < epi.kb0) tma_prefetch_2d_r<UNI>(&tm_a0, kb * BK, m1);
-            else tma_prefetch_2d_r<UNI>(&tm_a1, (kb - epi.kb0) * BK, m1);
-          }
-          if (cs == 1) {
-            tma_load_2d_r<UNI>(sa + A_BYTES, &tm_w, kb * BK, n_idx * BN, full_bar(stage));
-          } else {
-            const int rows = BN / int(cs);      // this CTA's slice of the weight tile, broadcast to the cluster
-            tma_load_2d_mc_r<UNI>(sa + A_BYTES + uint32_t(crank) * uint32_t(rows * BK * 2), &tm_w, kb * BK,
-                                  n_idx * BN + int(crank) * rows, full_bar(stage), cmask);
-          }
-          if (++stage == nst) { stage = 0; phase ^= 1u; }
+    // TMA producer: the whole warp walks the loop, one elected lane issues (see tc_common.cuh)
+    int stage = 0;
+    uint32_t phase = 0;
+    unsigned long long tw = 0, tstart = clock64();
+    for (int unit = cluster_id; unit < total; unit += num_clusters) {
+      const int tile = unit % tiles_mn, kb_lo = (unit / tiles_mn) * kb_per, kb_hi = min(kblocks, kb_lo + kb_per);
+      const int n_idx = tile % num_n, m_idx = (tile / num_n) * int(cs) + int(crank);   // N fastest: neighbours share A in L2
+      const int m0 = m_idx * epi.tile_rows;
+      for (int kb = kb_lo; kb < kb_hi; ++kb) {
+        unsigned long long t0 = epi.trace ? clock64() : 0;
+        mbar_wait(empty_bar(stage), phase ^ 1u, err_flag, 1);
+        if (epi.trace) tw += clock64() - t0;
+        const uint32_t sa = base + stage * stb;
+        if constexpr (TWO) {      // CTA pair: own token tile + own half of the weight tile, bytes counted on the leader
+          if (crank == 0) mbar_expect_tx_elect(full_bar(stage), Cfg::STAGE_TX_2SM);
+          if (kb < epi.kb0) tma_load_2d_2sm_elect(sa, &tm_a0, kb * BK, m0, full_bar(stage));
+          else tma_load_2d_2sm_elect(sa, &tm_a1, (kb - epi.kb0) * BK, m0, full_bar(stage));
+          tma_load_2d_2sm_elect(sa + A_BYTES, &tm_w, kb * BK, n_idx * BN + int(crank) * (BN / 2), full_bar(stage));
+        } else {
+          mbar_expect_tx_elect(full_bar(stage), Cfg::STAGE_BYTES);
+          if (kb < epi.kb0) tma_load_2d_elect(sa, &tm_a0, kb * BK, m0, full_bar(stage));
+          else tma_load_2d_elect(sa, &tm_a1, (kb - epi.kb0) * BK, m0, full_bar(stage));
+          tma_load_2d_elect(sa + A_BYTES, &tm_w, kb * BK, n_idx * BN, full_bar(stage));
         }
+        if (++stage == nst) { stage = 0; phase ^= 1u; }
       }
-      if (epi.trace && lane == 0) {
-        epi.trace[blockIdx.x * 8 + 0] = tw;
-        epi.trace[blockIdx.x * 8 + 1] = clock64() - tstart;
-      }
-    };
-    if (epi.uni_issue) producer(std::true_type{});
-    else producer(std::false_type{});
+    }
+    if (epi.trace && lane == 0) {
+      epi.trace[blockIdx.x * 8 + 0] = tw;
+      epi.trace[blockIdx.x * 8 + 1] = clock64() - tstart;
+    }
   } else if (warp == 1) {
-    // MMA issuer
-    auto issuer = [&](auto uni_tag) {
-      constexpr bool UNI = decltype(uni_tag)::value;
-      if (!UNI && lane != 0) return;
-      if (TWO && crank != 0) return;                 // CTA pair: the even CTA issues for both
+    // MMA issuer (CTA pair: the even CTA issues for both)
+    if (!TWO || crank == 0) {
       int stage = 0;
       uint32_t phase = 0;
       int ab = 0;
@@ -281,25 +253,22 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant__ CUt
           const uint32_t sa = base + stage * stb;
           const uint64_t adesc = umma_desc(sa, epi.desc_hi);
           const uint64_t bdesc = umma_desc(sa + A_BYTES, epi.desc_hi);
-          if constexpr (UNI && TWO) {
+          // advance 16 elements (32 bytes) along K inside the 128-byte swizzle row: +2 in 16-byte units
+          if constexpr (TWO) {
 #pragma unroll
             for (int k = 0; k < BK / 16; ++k)
               umma_issue_2sm_elect(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), Cfg::IDESC_2SM, ((kb - kb_lo) | k) != 0);
             umma_arrive_2sm_mc_elect(empty_bar(stage), 3);     // the slot is free in BOTH CTAs
-            if (++stage == nst) { stage = 0; phase ^= 1u; }
-            continue;
-          }
+          } else {
 #pragma unroll
-          for (int k = 0; k < BK / 16; ++k) {
-            // advance 16 elements (32 bytes) along K inside the 128-byte swizzle row: +2 in 16-byte units
-            umma_issue<UNI>(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), epi.idesc, ((kb - kb_lo) | k) != 0);
+            for (int k = 0; k < BK / 16; ++k)
+              umma_issue_elect(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), epi.idesc, ((kb - kb_lo) | k) != 0);
+            umma_arrive_elect(empty_bar(stage));     // smem slot reusable once these MMAs have read it
           }
-          if (cs == 1) umma_arrive<UNI>(empty_bar(stage));     // smem slot reusable once these MMAs have read it
-          else umma_arrive_mc<UNI>(empty_bar(stage), cmask);   // ... in every CTA of the cluster
           if (++stage == nst) { stage = 0; phase ^= 1u; }
         }
-        if constexpr (UNI && TWO) umma_arrive_2sm_mc_elect(tfull_bar(ab), 3);     // both CTAs' halves are complete
-        else umma_arrive<UNI>(tfull_bar(ab));               // accumulator complete -> epilogue
+        if constexpr (TWO) umma_arrive_2sm_mc_elect(tfull_bar(ab), 3);     // both CTAs' halves are complete
+        else umma_arrive_elect(tfull_bar(ab));               // accumulator complete -> epilogue
         if (++ab == 2) { ab = 0; aphase ^= 1u; }
       }
       if (epi.trace && lane == 0) {
@@ -307,9 +276,7 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant__ CUt
         epi.trace[blockIdx.x * 8 + 3] = tw_f;
         epi.trace[blockIdx.x * 8 + 4] = clock64() - tstart;
       }
-    };
-    if (epi.uni_issue) issuer(std::true_type{});
-    else issuer(std::false_type{});
+    }
   } else {
     // ---------------- epilogue warps ----------------
     const int q = warp & 3;                        // TMEM lane quadrant this warp may access
@@ -699,11 +666,10 @@ k_gemm_tc(const __grid_constant__ CUtensorMap tm_a0, const __grid_constant__ CUt
 // lanes of a warp to hold the channels in the order 8 (lane % 4) + lane / 4.  The host stores the weight rows of
 // these convs in exactly that order inside every block of 32 (ds_commit_weights), so the shuffle costs nothing.
 // GroupNorm statistics: per-(scene, channel) partials -> shared memory -> 8 threads per (scene, group) reduce.
-template <int NOBJ, bool PAIR = true, int SC_ = 0, bool SP = false>
+template <int NOBJ, bool PAIR = true>
 struct GntCfg {
-  // scenes per tile: 16 for N = 12 (UMMA N = 192), 12 for N = 21 (252 -> 256); SC_ = 20 selects 240-token tiles for
-  // N = 12 (an N = 192 MMA measures about the cycles of an N = 256 one, so wider tiles use the tensor pipe better)
-  static constexpr int SC = SC_ > 0 ? SC_ : ((NOBJ == 12) ? 16 : 256 / NOBJ);
+  // scenes per tile: 16 for N = 12 (UMMA N = 192), 12 for N = 21 (252 -> 256)
+  static constexpr int SC = (NOBJ == 12) ? 16 : 256 / NOBJ;
   static constexpr int TOK = SC * NOBJ;                         // tokens per tile (192 / 252)
   static constexpr int UN = (TOK + 15) / 16 * 16;               // UMMA N = TMA box rows of the activation tile
   static constexpr int EPI_W = 16;                              // epilogue warps: 4 per TMEM lane quadrant
@@ -712,10 +678,7 @@ struct GntCfg {
   static constexpr int THREADS = 64 + EPI_W * 32;
   static constexpr int B_BYTES = UN * BK * 2;
   static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  // SP ("spill") variant: the statistics pass parks the bf16-rounded accumulator of the warp's scenes in shared memory
-  // (lane-contiguous words, no bank conflicts, private to the thread that wrote them) so that the accumulator is read
-  // from TMEM only once and released before the normalisation pass; costs one pipeline stage of shared memory
-  static constexpr int STAGES = (UN <= 192) ? (SP ? 3 : 4) : 3;
+  static constexpr int STAGES = (UN <= 192) ? 4 : 3;
   static constexpr int ACC_STRIDE = 256;                        // TMEM columns between the two accumulators
   static constexpr int TMEM_COLS = 512;
   static constexpr int CHAN_MAX_N = 512;
@@ -737,10 +700,7 @@ struct GntCfg {
   static constexpr int RED_OFF = SCRATCH_OFF + CHAN_BYTES;
   static constexpr int STAT_OFF = RED_OFF + RED_BYTES;
   static constexpr int STG_OFF = (STAT_OFF + STAT_BYTES + 127) / 128 * 128;
-  static constexpr int SPILL_OFF = STG_OFF + EPI_W * 2 * STG_BYTES;
-  // [warp][scene][pair][lane] words; the warp's last scene stays in registers
-  static constexpr int SPILL_BYTES = SP ? EPI_W * (SPP - 1) * NPAIR * 128 : 0;
-  static constexpr int SMEM_BYTES = 1024 + SPILL_OFF + SPILL_BYTES;
+  static constexpr int SMEM_BYTES = 1024 + STG_OFF + EPI_W * 2 * STG_BYTES;
   static_assert(SC % NP == 0, "scenes must split evenly over the warps of a quadrant");
   static_assert(STAGE_BYTES % 1024 == 0, "stages must stay swizzle-atom aligned");
   static_assert(SMEM_BYTES <= 232448, "shared memory budget exceeded");
@@ -824,14 +784,13 @@ __device__ __forceinline__ void stsm_x2_t(uint32_t addr, uint32_t r0, uint32_t r
 
 // TWO: the CTA-pair instantiation (cta_group::2 instructions; must be launched with a cluster of 2 -- the driver
 // refuses a plain launch of a kernel that contains them, so the single-CTA path is a separate instantiation)
-template <int NOBJ, bool PAIR, int SC_, bool SP, bool TWO = false>
+template <int NOBJ, bool PAIR, bool TWO = false>
 // 18 warps = 5 on the fullest SM sub-partition: 16384 / (5 * 32) = 102 registers per thread at most
 __global__ void __maxnreg__(96)
 k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_x0,
            const __grid_constant__ CUtensorMap tm_x1, TcEpi epi, int* err_flag) {
-  using Cfg = GntCfg<NOBJ, PAIR, SC_, SP>;
+  using Cfg = GntCfg<NOBJ, PAIR>;
   static_assert(!PAIR || Cfg::SPP <= 4, "the warp-pair statistics exchange packs at most 4 scenes per warp");
-  static_assert(!SP || (!PAIR && NOBJ % 2 == 0), "the spill variant is written for the default statistics path and even N");
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* const base_ptr = smem_raw + (base - smem_u32(smem_raw));
@@ -853,13 +812,9 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
 
   const int warp = uniform_warp_idx(), lane = threadIdx.x & 31;
   asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-  // Optional thread-block cluster (DS_GNT_CLUSTER=2): the CS CTAs of a cluster work on CS channel tiles of the SAME
-  // token tile and share the activation tile -- each CTA loads 1 / CS of its rows and multicasts the slice into every
-  // CTA's shared memory, which cuts the L2 -> SM operand stream (320 KB per tile) by 30 % at CS = 2.
   const uint32_t cs = cluster_nctarank();
   const uint32_t crank = cluster_ctarank();
-  const uint16_t cmask = uint16_t((1u << cs) - 1u);
-  // CTA-pair mode (DS_GNT_2CTA=1, cluster of 2): ONE tcgen05.mma.cta_group::2 of M = 256 covers both CTAs' channel tiles
+  // CTA pair (TWO, cluster of 2): ONE tcgen05.mma.cta_group::2 of M = 256 covers both CTAs' channel tiles
   // of the same token tile.  Each CTA loads its own weight tile and HALF of the token tile (224 KB instead of 320 KB
   // from L2 per tile pair-half, and the tensor core reads 7 KB instead of 10 KB of shared memory per MMA and SM); the
   // even CTA issues the MMAs for the pair, and every pipeline barrier that gates them lives in that CTA:
@@ -867,23 +822,21 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
   //   empty[s]   both CTAs: 1 arrival each from the leader's multicast commit
   //   tfull[b]   both CTAs: 1 arrival each from the leader's multicast commit
   //   tempty[b]  leader only: 2 x 16 arrivals (the epilogue warps of both CTAs)
-  constexpr bool two = TWO;
   // operand ring geometry: the CTA pair stages only half of the token tile per CTA, so the same shared memory holds
   // more (smaller) stages
-  const bool deep = two && !(epi.two_cta & 4);         // DS_GNT_2CTA |= 4: keep the single-CTA ring geometry (A/B)
-  const int nst = deep ? Cfg::STAGES_2SM : Cfg::STAGES;
-  const uint32_t stb = deep ? uint32_t(Cfg::STAGE_BYTES_2SM) : uint32_t(Cfg::STAGE_BYTES);
+  constexpr int nst = TWO ? Cfg::STAGES_2SM : Cfg::STAGES;
+  constexpr uint32_t stb = TWO ? uint32_t(Cfg::STAGE_BYTES_2SM) : uint32_t(Cfg::STAGE_BYTES);
   if (warp == 0 && lane == 0) {
     tma_prefetch_desc(&tm_w);
     tma_prefetch_desc(&tm_x0);
     tma_prefetch_desc(&tm_x1);
     for (int s = 0; s < Cfg::MAX_STAGES; ++s) {
       mbar_init(full_bar(s), 1);
-      mbar_init(empty_bar(s), two ? 1 : cs);       // multicast mode: every CTA of the cluster must have consumed the slot
+      mbar_init(empty_bar(s), 1);
     }
     for (int b = 0; b < 2; ++b) {
       mbar_init(tfull_bar(b), 1);
-      mbar_init(tempty_bar(b), two ? 2 * Cfg::EPI_W : Cfg::EPI_W);
+      mbar_init(tempty_bar(b), TWO ? 2 * Cfg::EPI_W : Cfg::EPI_W);
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -911,7 +864,7 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
   const int n_scenes_total = epi.M / NOBJ;
   const int num_tt = (n_scenes_total + Cfg::SC - 1) / Cfg::SC;     // token tiles
   const int num_ct = epi.N / BM;                                    // channel tiles
-  // work units: (token tile, group of CS channel tiles); the CTAs of a cluster walk the same unit sequence and
+  // work units: (token tile, group of CS channel tiles); the CTAs of a pair walk the same unit sequence and
   // CTA `crank` takes channel tile group * CS + crank.  CS == 1: unit == tile, exactly the single-CTA schedule.
   const int cgn = num_ct / int(cs);
   const int total = num_tt * cgn;
@@ -919,63 +872,39 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
   const int kblocks = epi.kb0 + epi.kb1;
 
   if (warp == 0) {
-    // TMA producer.  UNI: the whole warp walks the loop, one elected lane issues (see tc_common.cuh)
-    auto producer = [&](auto uni_tag) {
-      constexpr bool UNI = decltype(uni_tag)::value;
-      if (!UNI && lane != 0) return;
-      int stage = 0;
-      uint32_t phase = 0;
-      unsigned long long tw = 0, tstart = clock64();
-      for (int tile = unit0; tile < total; tile += unit_step) {
-        const int ct = (tile % cgn) * int(cs) + int(crank), tt = tile / cgn;   // channel tiles fastest: neighbours share X
-        const int m0 = tt * Cfg::TOK;
-        for (int kb = 0; kb < kblocks; ++kb) {
-          unsigned long long t0 = epi.trace ? clock64() : 0;
-          mbar_wait(empty_bar(stage), phase ^ 1u, err_flag, 1);
-          if (epi.trace) tw += clock64() - t0;
-          const uint32_t sa = base + stage * stb;
-          const CUtensorMap* tmx = kb < epi.kb0 ? &tm_x0 : &tm_x1;
-          const int kx = (kb < epi.kb0 ? kb : kb - epi.kb0) * BK;
-          if constexpr (UNI && TWO) {
-            {               // CTA pair: own weight tile + own half of the token tile, bytes counted on the leader's barrier
-              if (crank == 0) mbar_expect_tx_r<true>(full_bar(stage), Cfg::STAGE_TX_2SM);
-              tma_load_2d_2sm_elect(sa, &tm_w, kb * BK, ct * BM, full_bar(stage));
-              tma_load_2d_2sm_elect(sa + A_BYTES, tmx, kx, m0 + int(crank) * (Cfg::UN / 2),
-                                    full_bar(stage));
-              if (++stage == nst) { stage = 0; phase ^= 1u; }
-              continue;
-            }
-          }
-          mbar_expect_tx_r<UNI>(full_bar(stage), Cfg::STAGE_BYTES);
-          tma_load_2d_r<UNI>(sa, &tm_w, kb * BK, ct * BM, full_bar(stage));
-          if (cs == 1) {
-            tma_load_2d_r<UNI>(sa + A_BYTES, tmx, kx, m0, full_bar(stage));
-            // DS_TC_L2PF: pull the NEXT token tile of this CTA towards L2 a whole tile time ahead (the activations were
-            // written by the previous kernel and are only partly L2-resident); the channel-tile-0 CTA does it for the
-            // CTAs that share the token tile
-            if (epi.l2_prefetch && ct == 0 && tile + unit_step < total)
-              tma_prefetch_2d_r<UNI>(tmx, kx, ((tile + unit_step) / cgn) * Cfg::TOK);
-          } else {
-            const int rows = Cfg::UN / int(cs);      // this CTA's slice of the activation tile, broadcast to the cluster
-            tma_load_2d_mc_r<UNI>(sa + A_BYTES + uint32_t(crank) * uint32_t(rows * BK * 2), tmx, kx, m0 + int(crank) * rows,
-                                  full_bar(stage), cmask);
-          }
-          if (++stage == nst) { stage = 0; phase ^= 1u; }
+    // TMA producer: the whole warp walks the loop, one elected lane issues (see tc_common.cuh)
+    int stage = 0;
+    uint32_t phase = 0;
+    unsigned long long tw = 0, tstart = clock64();
+    for (int tile = unit0; tile < total; tile += unit_step) {
+      const int ct = (tile % cgn) * int(cs) + int(crank), tt = tile / cgn;   // channel tiles fastest: neighbours share X
+      const int m0 = tt * Cfg::TOK;
+      for (int kb = 0; kb < kblocks; ++kb) {
+        unsigned long long t0 = epi.trace ? clock64() : 0;
+        mbar_wait(empty_bar(stage), phase ^ 1u, err_flag, 1);
+        if (epi.trace) tw += clock64() - t0;
+        const uint32_t sa = base + stage * stb;
+        const CUtensorMap* tmx = kb < epi.kb0 ? &tm_x0 : &tm_x1;
+        const int kx = (kb < epi.kb0 ? kb : kb - epi.kb0) * BK;
+        if constexpr (TWO) {      // CTA pair: own weight tile + own half of the token tile, bytes counted on the leader's barrier
+          if (crank == 0) mbar_expect_tx_elect(full_bar(stage), Cfg::STAGE_TX_2SM);
+          tma_load_2d_2sm_elect(sa, &tm_w, kb * BK, ct * BM, full_bar(stage));
+          tma_load_2d_2sm_elect(sa + A_BYTES, tmx, kx, m0 + int(crank) * (Cfg::UN / 2), full_bar(stage));
+        } else {
+          mbar_expect_tx_elect(full_bar(stage), Cfg::STAGE_BYTES);
+          tma_load_2d_elect(sa, &tm_w, kb * BK, ct * BM, full_bar(stage));
+          tma_load_2d_elect(sa + A_BYTES, tmx, kx, m0, full_bar(stage));
         }
+        if (++stage == nst) { stage = 0; phase ^= 1u; }
       }
-      if (epi.trace && lane == 0) {
-        epi.trace[blockIdx.x * 8 + 0] = tw;
-        epi.trace[blockIdx.x * 8 + 1] = clock64() - tstart;
-      }
-    };
-    if (epi.uni_issue) producer(std::true_type{});
-    else producer(std::false_type{});
+    }
+    if (epi.trace && lane == 0) {
+      epi.trace[blockIdx.x * 8 + 0] = tw;
+      epi.trace[blockIdx.x * 8 + 1] = clock64() - tstart;
+    }
   } else if (warp == 1) {
-    // MMA issuer
-    auto issuer = [&](auto uni_tag) {
-      constexpr bool UNI = decltype(uni_tag)::value;
-      if (!UNI && lane != 0) return;
-      if (two && crank != 0) return;                 // CTA pair: the even CTA issues for both
+    // MMA issuer (CTA pair: the even CTA issues for both)
+    if (!TWO || crank == 0) {
       int stage = 0;
       uint32_t phase = 0;
       int ab = 0;
@@ -995,25 +924,21 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
           const uint32_t sa = base + stage * stb;
           const uint64_t adesc = umma_desc(sa, epi.desc_hi);                // weights: the M operand
           const uint64_t bdesc = umma_desc(sa + A_BYTES, epi.desc_hi);      // activations: the N operand
-          if constexpr (UNI && TWO) {
-            {
+          if constexpr (TWO) {
 #pragma unroll
-              for (int k = 0; k < BK / 16; ++k)
-                umma_issue_2sm_elect(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), Cfg::IDESC_2SM, (kb | k) != 0);
-              umma_arrive_2sm_mc_elect(empty_bar(stage), 3);     // the slot is free in BOTH CTAs
-              if (++stage == nst) { stage = 0; phase ^= 1u; }
-              continue;
-            }
+            for (int k = 0; k < BK / 16; ++k)
+              umma_issue_2sm_elect(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), Cfg::IDESC_2SM, (kb | k) != 0);
+            umma_arrive_2sm_mc_elect(empty_bar(stage), 3);     // the slot is free in BOTH CTAs
+          } else {
+#pragma unroll
+            for (int k = 0; k < BK / 16; ++k)
+              umma_issue_elect(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), Cfg::IDESC, (kb | k) != 0);
+            umma_arrive_elect(empty_bar(stage));     // smem slot reusable once these MMAs have read it
           }
-#pragma unroll
-          for (int k = 0; k < BK / 16; ++k)
-            umma_issue<UNI>(d_tmem, adesc + uint64_t(2 * k), bdesc + uint64_t(2 * k), Cfg::IDESC, (kb | k) != 0);
-          if (cs == 1) umma_arrive<UNI>(empty_bar(stage));     // smem slot reusable once these MMAs have read it
-          else umma_arrive_mc<UNI>(empty_bar(stage), cmask);   // ... in every CTA of the cluster
           if (++stage == nst) { stage = 0; phase ^= 1u; }
         }
-        if constexpr (UNI && TWO) umma_arrive_2sm_mc_elect(tfull_bar(ab), 3);     // both CTAs' halves of the accumulator are complete
-        else umma_arrive<UNI>(tfull_bar(ab));
+        if constexpr (TWO) umma_arrive_2sm_mc_elect(tfull_bar(ab), 3);     // both CTAs' halves of the accumulator are complete
+        else umma_arrive_elect(tfull_bar(ab));
         if (++ab == 2) { ab = 0; aphase ^= 1u; }
       }
       if (epi.trace && lane == 0) {
@@ -1021,9 +946,7 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
         epi.trace[blockIdx.x * 8 + 3] = tw_f;
         epi.trace[blockIdx.x * 8 + 4] = clock64() - tstart;
       }
-    };
-    if (epi.uni_issue) issuer(std::true_type{});
-    else issuer(std::false_type{});
+    }
   } else {
     // ---------------- epilogue warps ----------------
     auto epi_bar = []() { asm volatile("bar.sync 1, %0;" ::"n"(Cfg::EPI_W * 32) : "memory"); };
@@ -1046,9 +969,6 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
     // staging blocks of this warp: [token][32 channels] bf16, 64 B rows
     const uint32_t stg_in = base + uint32_t(Cfg::STG_OFF) + uint32_t((warp - 2) * 2 * Cfg::STG_BYTES);
     const uint32_t stg_out = stg_in + uint32_t(Cfg::STG_BYTES);
-    // spill words of this thread (SP variant only): [scene][pair][lane]
-    uint32_t* const spill = reinterpret_cast<uint32_t*>(base_ptr + Cfg::SPILL_OFF) + (warp - 2) * ((Cfg::SPP - 1) * Cfg::NPAIR * 32) + lane;
-    uint32_t keep[SP ? Cfg::NPAIR : 1];               // packed values of the warp's last scene (SP variant)
     // ldmatrix / stmatrix row address of this lane: matrix lane / 8 holds tokens 2 (lane / 8) + {0, 1}; its row
     // (lane % 8) = 2 * chunk + e is the 16-byte chunk `chunk` (8 channels) of token 2 (lane / 8) + e
     const uint32_t mrow = uint32_t((2 * (lane >> 3) + (lane & 1)) * 64 + ((lane & 7) >> 1) * 16);
@@ -1125,23 +1045,6 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
         };
         if constexpr (RES) {
           if (0 < n_live) fetch_res();
-          // Pull the NEXT tile's residual rows of this warp towards L2 now, a whole tile time ahead of their use: the
-          // per-scene fetches in pass 2 then hit L2 instead of waiting on HBM (the largest single stall of this
-          // kernel in the round-1 profile).  The very first tile of a CTA prefetches its own rows as well.
-          auto prefetch_rows = [&](int p_tt, int p_ct) {
-            const int p_scene0 = p_tt * Cfg::SC + s_begin;
-            const char* pp = reinterpret_cast<const char*>(epi.res + ((int64_t)p_scene0 * NOBJ + lane) * epi.ldres + p_ct * BM + 32 * q);
-            const int rows_left = epi.M - p_scene0 * NOBJ;
-            if (lane < Cfg::SPP * NOBJ && lane < rows_left) asm volatile("prefetch.global.L2 [%0];" ::"l"(pp));
-            if (lane + 32 < Cfg::SPP * NOBJ && lane + 32 < rows_left)
-              asm volatile("prefetch.global.L2 [%0];" ::"l"(pp + (int64_t)32 * epi.ldres * 2));
-          };
-          if (epi.res_prefetch && tile == unit0) prefetch_rows(tt, ct);
-          if (epi.res_prefetch && tile + unit_step < total) {
-            int ncg = cg + step_cg, ntt = tt + step_tt;
-            if (ncg >= cgn) { ncg -= cgn; ++ntt; }
-            prefetch_rows(ntt, ncg * int(cs) + int(crank));
-          }
         }
         unsigned long long t0 = epi.trace ? clock64() : 0;
         mbar_wait(tfull_bar(ab), aphase, err_flag, 4);
@@ -1208,38 +1111,7 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
 
         } else {
         // ---- pass 1: per-(scene, channel) sums of acc and acc^2 over the scene's tokens, bias folded analytically
-        if constexpr (FM != 4 && NOBJ == 12 && Cfg::SPP == 4 && !SP) {
-          // all four scenes of this warp (48 accumulator columns) with two wide TMEM loads instead of eight narrow ones
-          // (DS_GNT_WIDE1=0 selects the per-scene loads; A/B in profiles/)
-          if (epi.wide_pass1) {
-            uint32_t w32[32], w16[16];
-            tmem_ld32_issue(taddr, w32);
-            asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-                         "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                         : "=r"(w16[0]), "=r"(w16[1]), "=r"(w16[2]), "=r"(w16[3]), "=r"(w16[4]), "=r"(w16[5]), "=r"(w16[6]),
-                           "=r"(w16[7]), "=r"(w16[8]), "=r"(w16[9]), "=r"(w16[10]), "=r"(w16[11]), "=r"(w16[12]),
-                           "=r"(w16[13]), "=r"(w16[14]), "=r"(w16[15])
-                         : "r"(taddr + 32u)
-                         : "memory");
-            tmem_ld_wait();
-            float2* rdst = red + s_begin * 128 + 32 * q + lane;
-#pragma unroll
-            for (int si = 0; si < 4; ++si) {
-              float s1 = 0.f, s2 = 0.f;
-#pragma unroll
-              for (int j = 0; j < 12; ++j) {
-                const int col = si * 12 + j;
-                const float v = __uint_as_float(col < 32 ? w32[col < 32 ? col : 0] : w16[col >= 32 ? col - 32 : 0]);
-                s1 += v;
-                s2 = fmaf(v, v, s2);
-              }
-              const float S = fmaf(12.0f, bias, s1);
-              const float SS = fmaf(bias, fmaf(12.0f, bias, 2.0f * s1), s2);
-              rdst[si * 128] = make_float2(S, SS);
-            }
-          }
-        }
-        if (FM != 4 && !(NOBJ == 12 && Cfg::SPP == 4 && !SP && epi.wide_pass1)) {
+        if constexpr (FM != 4) {
           uint32_t va[NOBJ];
           tmem_ld_scene_issue(taddr, va);
           float2* rdst = red + s_begin * 128 + 32 * q + lane;
@@ -1259,19 +1131,6 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
             const float S = fmaf(float(NOBJ), bias, s1);
             const float SS = fmaf(bias, fmaf(float(NOBJ), bias, 2.0f * s1), s2);
             rdst[si * 128] = make_float2(S, SS);
-            if constexpr (SP) {
-#pragma unroll
-              for (int i = 0; i < Cfg::NPAIR; ++i) {
-                __nv_bfloat162 h2 = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
-                if (si + 1 < Cfg::SPP) spill[(si * Cfg::NPAIR + i) * 32] = *reinterpret_cast<uint32_t*>(&h2);
-                else keep[i] = *reinterpret_cast<uint32_t*>(&h2);
-              }
-            }
-          }
-          if constexpr (SP) {      // the accumulator has been read: the next-but-one tile's MMAs may start already
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) { if constexpr (TWO) mbar_arrive_leader(tempty_bar(ab)); else mbar_arrive(tempty_bar(ab)); }
           }
         }
         if constexpr (FM != 4) epi_bar();
@@ -1333,14 +1192,6 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
           float y[2 * Cfg::PKN];                      // tokens >= NOBJ: padding of the last pair(s), never stored
 #pragma unroll
           for (int j = NOBJ; j < 2 * Cfg::PKN; ++j) y[j] = 0.f;
-          if constexpr (SP && FM != 4) {              // values parked by pass 1; TMEM was released there
-#pragma unroll
-            for (int i = 0; i < Cfg::NPAIR; ++i) {
-              const uint32_t w = si + 1 < Cfg::SPP ? spill[(si * Cfg::NPAIR + i) * 32] : keep[i];
-              y[2 * i] = fmaf(__uint_as_float(w << 16), a, b);
-              y[2 * i + 1] = fmaf(__uint_as_float(w & 0xffff0000u), a, b);
-            }
-          } else {
           tmem_ld_scene_wait(va);
 #pragma unroll
           for (int j = 0; j < NOBJ; ++j) y[j] = FM == 4 ? __uint_as_float(va[j]) + b : fmaf(__uint_as_float(va[j]), a, b);
@@ -1350,7 +1201,6 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
             __syncwarp();
             // accumulator drained: the next tile's MMAs may start (CTA pair: counted on the leader's barrier)
             if (lane == 0) { if constexpr (TWO) mbar_arrive_leader(tempty_bar(ab)); else mbar_arrive(tempty_bar(ab)); }
-          }
           }
           if constexpr (FM == 1) {
             if constexpr (OBJ_IN_REGS) {
@@ -1486,8 +1336,6 @@ k_gemm_gnt(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUt
 // ------------------------------------------------------------------------------------------------
 // host side: tensor maps + launch
 // ------------------------------------------------------------------------------------------------
-static int gnt_two_cta();
-static constexpr int TC_2CTA_DEFAULT = 1;      // row-major kernel: CTA pair off / on by default (DS_TC_2CTA)
 struct TcGemmPlan {
   CUtensorMap tm_a0, tm_a1, tm_w;
   TcEpi epi;
@@ -1495,8 +1343,7 @@ struct TcGemmPlan {
   bool gn;
   bool gnt;          // GroupNorm epilogue, channels-on-lanes variant (weights stored in the permuted row order)
   int num_sms;
-  int cluster;       // CTAs per cluster (weight-tile multicast width): 1, 2 or 4
-  int max_clusters;  // co-resident clusters of that size
+  int cluster;       // CTAs per cluster: 1, or 2 for the CTA pair (TWO instantiations)
 };
 
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -1532,17 +1379,10 @@ bool tc_runtime_available(char* err, int err_len) {
   cudaFuncSetAttribute(k_gemm_tc<256, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256, false>::SMEM_BYTES);
   cudaFuncSetAttribute(k_gemm_tc<256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256, true>::SMEM_BYTES);
   cudaFuncSetAttribute(k_gemm_tc<256, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcCfg<256, false>::SMEM_BYTES);
-  cudaFuncSetAttribute(k_gemm_gnt<12, true, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<12, true>::SMEM_BYTES);
-  cudaFuncSetAttribute(k_gemm_gnt<21, true, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<21, true>::SMEM_BYTES);
-  cudaFuncSetAttribute(k_gemm_gnt<12, false, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<12, false>::SMEM_BYTES);
-  cudaFuncSetAttribute(k_gemm_gnt<21, false, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<21, false>::SMEM_BYTES);
-  cudaFuncSetAttribute(k_gemm_gnt<12, false, 20, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<12, false, 20>::SMEM_BYTES);
-  cudaFuncSetAttribute(k_gemm_gnt<12, false, 0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<12, false>::SMEM_BYTES);
-  cudaFuncSetAttribute(k_gemm_gnt<21, false, 0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<21, false>::SMEM_BYTES);
-  cudaFuncSetAttribute(k_gemm_gnt<12, false, 0, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<12, false, 0, true>::SMEM_BYTES);
-  cudaFuncSetAttribute(k_gemm_gnt<12, true, 0, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<12, true>::SMEM_BYTES);
-  cudaFuncSetAttribute(k_gemm_gnt<12, false, 0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                       GntCfg<12, false, 0, true>::SMEM_BYTES);
+  cudaFuncSetAttribute(k_gemm_gnt<12, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<12, true>::SMEM_BYTES);
+  cudaFuncSetAttribute(k_gemm_gnt<21, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<21, true>::SMEM_BYTES);
+  cudaFuncSetAttribute(k_gemm_gnt<12, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<12, true>::SMEM_BYTES);
+  cudaFuncSetAttribute(k_gemm_gnt<21, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, GntCfg<21, false>::SMEM_BYTES);
   g_encode = (PFN_encodeTiled)fn;
   return true;
 }
@@ -1564,12 +1404,6 @@ static bool encode_2d(CUtensorMap* map, const void* base, uint64_t inner, uint64
     return false;
   }
   return true;
-}
-
-// scenes per tile of the channels-on-lanes kernel for N = 12: 16 (default) or 20 (DS_GNT_SC=20, A/B switch)
-static int gnt_scenes_per_tile(int n_obj) {
-  static const int sc = getenv("DS_GNT_SC") ? atoi(getenv("DS_GNT_SC")) : 16;
-  return n_obj == 12 ? (sc == 20 ? 20 : 16) : 12;
 }
 
 TcGemmPlan* tc_plan_create(const GemmArgs& g, int rows_capacity, char* err, int err_len) {
@@ -1611,47 +1445,24 @@ TcGemmPlan* tc_plan_create(const GemmArgs& g, int rows_capacity, char* err, int 
   p->gn = gn;
   p->gnt = gnt;
   p->num_sms = g_num_sms;
-  // channels-on-lanes kernel: optional cluster of 2 CTAs sharing the activation tile (each loads half, multicast)
-  int gnt_cs = 1;
-  if (gnt) {
-    if (const char* e = getenv("DS_GNT_CLUSTER")) gnt_cs = atoi(e);
-  }
-  const int gnt_sc20 = gnt_scenes_per_tile(g.n_obj) == 20;
-  // CTA-pair MMAs (cta_group::2): DS_GNT_2CTA = 0 off, 1 wherever the shape allows, 2 (default) for K >= 1024 only --
-  // measured on B200 (profiles/round2_probe_2cta.txt): the K = 1024 skip convs gain 15 % (66.3 -> 56.6 us), the
-  // K = 512 blocks do not (39.2 us either way; with a residual the pair's lock-step costs 3 us)
-  int two_cta = 0;
-  if (gnt && !gnt_sc20 && tc_uniform_issue() && (g.N / BM) % 2 == 0) {
-    const int mode = gnt_two_cta() & 3;
-    if (mode == 1 || (mode == 2 && K >= 1024)) two_cta = 1 | (gnt_two_cta() & 4);
-  }
-  if (gnt) {
-    if (two_cta) gnt_cs = 2;                       // the pair is a cluster of 2
-    if (gnt_cs != 2 || (g.N / BM) % 2 != 0) gnt_cs = 1;
-  }
-  // row-major plain kernel, 128 x 256 tiles: DS_TC_2CTA = 0 off, 1 (default) CTA pair where it measured faster --
-  // K >= DS_TC_2CTA_K (1024) or N >= DS_TC_2CTA_N (2048).  Same box, 4096 scenes (profiles/round2_probe_tc2.txt):
-  // 512 x 1024 51.0 -> 45.1 us, encoder K = 3072 128.3 -> 119.6 us, dec.l0 N = 3072 143.3 -> 137.1 us, but
-  // 512 x 512 31.2 -> 34.2 us and enc.l1 (N = 1024, K = 512) 51.4 -> 52.5 us; whole sample +1.4 % with the pair on
-  // every K >= 256 launch.  All 111 GPU tests ran green with the pair on every K >= 256 launch (a superset).
-  int tc_two = 0;
-  if (!gnt && !gn && !g.no_pair && p->bn == 256 && tc_uniform_issue()) {
-    static const int m2 = getenv("DS_TC_2CTA") ? atoi(getenv("DS_TC_2CTA")) : TC_2CTA_DEFAULT;
-    static const int k2 = getenv("DS_TC_2CTA_K") ? atoi(getenv("DS_TC_2CTA_K")) : 1024;
-    static const int n2 = getenv("DS_TC_2CTA_N") ? atoi(getenv("DS_TC_2CTA_N")) : 2048;
-    if (m2 && (K >= k2 || g.N >= n2)) tc_two = 1;
-  }
-  const int gnt_un = g.n_obj == 21 ? GntCfg<21, true>::UN : (gnt_sc20 ? GntCfg<12, false, 20>::UN : GntCfg<12, true>::UN);
-  const int gnt_tok = g.n_obj == 21 ? GntCfg<21, true>::TOK : (gnt_sc20 ? GntCfg<12, false, 20>::TOK : GntCfg<12, true>::TOK);
-  const uint32_t act_box = gnt ? uint32_t(gnt_un / gnt_cs) : uint32_t(BM);     // rows of one activation load
+  // CTA pair (cta_group::2, a cluster of 2): one M = 256 MMA spans two CTAs, each of which loads half of the operand
+  // they share.  Channels-on-lanes kernel: K >= 1024 and an even channel-tile count -- measured on B200
+  // (profiles/round2_probe_2cta.txt): the K = 1024 skip convs gain 15 % (66.3 -> 56.6 us), the K = 512 blocks do not
+  // (39.2 us either way; with a residual the pair's lock-step costs 3 us).
+  // Row-major plain kernel, 128 x 256 tiles: K >= 1024 or N >= 2048.  Same box, 4096 scenes
+  // (profiles/round2_probe_tc2.txt): 512 x 1024 51.0 -> 45.1 us, encoder K = 3072 128.3 -> 119.6 us, dec.l0 N = 3072
+  // 143.3 -> 137.1 us, but 512 x 512 31.2 -> 34.2 us and enc.l1 (N = 1024, K = 512) 51.4 -> 52.5 us; whole sample
+  // +1.4 % with the pair on every K >= 256 launch.  All 111 GPU tests ran green with the pair on every K >= 256 launch
+  // (a superset).
+  const bool two = gnt ? K >= 1024 && (g.N / BM) % 2 == 0
+                       : !gn && !g.no_pair && p->bn == 256 && (K >= 1024 || g.N >= 2048);
+  p->cluster = two ? 2 : 1;
+  const int gnt_un = g.n_obj == 21 ? GntCfg<21>::UN : GntCfg<12>::UN;
+  const int gnt_tok = g.n_obj == 21 ? GntCfg<21>::TOK : GntCfg<12>::TOK;
+  const uint32_t act_box = gnt ? uint32_t(gnt_un / p->cluster) : uint32_t(BM);     // rows of one activation load
   bool ok = encode_2d(&p->tm_a0, g.a0, g.k0, rows_capacity, g.lda0, act_box, err, err_len);
   if (ok && g.a1) ok = encode_2d(&p->tm_a1, g.a1, g.k1, rows_capacity, g.lda1, act_box, err, err_len);
   if (ok && !g.a1) p->tm_a1 = p->tm_a0;
-  p->cluster = 1;
-  if (const char* e = getenv("DS_TC_CLUSTER")) p->cluster = atoi(e);
-  if (p->cluster != 1 && p->cluster != 2 && p->cluster != 4) p->cluster = 1;
-  if (tc_two) p->cluster = 2;
-  if (gnt) p->cluster = gnt_cs;
   if (ok) ok = encode_2d(&p->tm_w, g.w, K, g.N, g.ldw, gnt ? BM : p->bn / p->cluster, err, err_len);
   const int tile_rows = gnt ? gnt_tok : (gn ? (BM / g.n_obj) * g.n_obj : BM);
   if (gn && !gnt && tile_rows / g.n_obj > TcCfg<256, true>::SPT_FAST) {
@@ -1684,21 +1495,6 @@ TcGemmPlan* tc_plan_create(const GemmArgs& g, int rows_capacity, char* err, int 
   p->epi.plain = plain_t ? 1 : 0;
   p->epi.d32 = nullptr;
   p->epi.ksplit = 1;
-  {
-    // measured (profiles/round2_gnt_ab.txt): the prefetch makes the residual variants 4-5 % SLOWER -- off by default
-    static const int pf = getenv("DS_GNT_PREFETCH") ? atoi(getenv("DS_GNT_PREFETCH")) : 0;
-    p->epi.res_prefetch = pf;
-    // measured (profiles/round2_gnt_ab.txt): no difference (39.1 vs 39.2 us) -> off
-    static const int wide = getenv("DS_GNT_WIDE1") ? atoi(getenv("DS_GNT_WIDE1")) : 0;
-    p->epi.wide_pass1 = wide;
-    p->epi.uni_issue = tc_uniform_issue();
-    static const int l2pf = getenv("DS_TC_L2PF") ? atoi(getenv("DS_TC_L2PF")) : 0;
-    p->epi.l2_prefetch = l2pf;
-    p->epi.two_cta = gnt ? ((gnt_cs == 2) ? two_cta : 0) : tc_two;
-  }
-  // bring-up overrides (hex), e.g. DS_TC_DESC_HI=0x4000404000010000
-  if (const char* e = getenv("DS_TC_DESC_HI")) p->epi.desc_hi = strtoull(e, nullptr, 16);
-  if (const char* e = getenv("DS_TC_IDESC")) p->epi.idesc = (uint32_t)strtoul(e, nullptr, 16);
   return p;
 }
 void tc_plan_destroy(TcGemmPlan* p) { delete p; }
@@ -1734,45 +1530,34 @@ static int launch_one(const TcGemmPlan* p, const TcEpi& epi, int total_ct, int* 
   cfg.numAttrs = 1;
   // off by default at the throughput batch: with the 576-thread channels-on-lanes kernels in the step program PDL
   // measured 1.5 % SLOWER (the chip is power-capped; early-resident CTAs polling their barriers cost clock)
-  const bool pdl = tc_pdl_enabled(epi.M);
+  const bool pdl = pdl_enabled(epi.M);
   if (pdl) {      // may start while the previous kernel in the stream drains (it waits at griddepcontrol.wait)
     attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[1].val.programmaticStreamSerializationAllowed = 1;
     cfg.numAttrs = 2;
   }
-  if (cs > 1) {
-    static int cached[4][5] = {{0}};      // [kernel variant][cluster size]
-    const int kv = TWO ? 3 : (GN ? 2 : (BN == 256 ? 1 : 0));
-    if (!cached[kv][cs]) {
-      cfg.gridDim = dim3(p->num_sms / cs * cs);
+  if constexpr (TWO) {
+    static int cached = 0;      // co-resident CTA pairs
+    if (!cached) {
+      cfg.gridDim = dim3(max_cl * cs);
       int n = 0;
-      if (cudaOccupancyMaxActiveClusters(&n, k_gemm_tc<BN, GN, TWO>, &cfg) == cudaSuccess && n > 0) cached[kv][cs] = n;
-      else cached[kv][cs] = max_cl;
+      cached = (cudaOccupancyMaxActiveClusters(&n, k_gemm_tc<BN, GN, TWO>, &cfg) == cudaSuccess && n > 0) ? n : max_cl;
     }
-    if (cached[kv][cs] < max_cl) max_cl = cached[kv][cs];
+    if (cached < max_cl) max_cl = cached;
   }
   const int ncl = total_ct < max_cl ? total_ct : max_cl;
   cfg.gridDim = dim3(ncl * cs);
   return (int)cudaLaunchKernelEx(&cfg, k_gemm_tc<BN, GN, TWO>, p->tm_a0, p->tm_a1, p->tm_w, epi, flag_dev);
 }
 
-// object counts the channels-on-lanes kernel is instantiated for (DS_GNT21=0 keeps N = 21 on the row-major kernel)
-static bool gnt_nobj_ok(int n_obj) {
-  static const int allow21 = getenv("DS_GNT21") ? atoi(getenv("DS_GNT21")) : 1;
-  return n_obj == 12 || (n_obj == 21 && allow21);
-}
+// object counts the channels-on-lanes kernel is instantiated for
+static bool gnt_nobj_ok(int n_obj) { return n_obj == 12 || n_obj == 21; }
 bool tc_gnt_plain_supported(int n_obj, int N) { return gnt_nobj_ok(n_obj) && N % BM == 0; }
 bool tc_gnt_supported(int n_obj, int N) { return gnt_nobj_ok(n_obj) && N % BM == 0 && N <= GntCfg<12, true>::CHAN_MAX_N; }
 
-// DS_GNT_2CTA: 0 off, 1 always, 2 by shape (default); | 4: keep the single-CTA operand-ring geometry (A/B)
-static int gnt_two_cta() {
-  static const int v = getenv("DS_GNT_2CTA") ? atoi(getenv("DS_GNT_2CTA")) : 2;
-  return v;
-}
-
-template <int NOBJ, bool PAIR, int SC_ = 0, bool SP = false, bool TWO = false>
+template <int NOBJ, bool PAIR, bool TWO = false>
 static int launch_gnt(const TcGemmPlan* p, const TcEpi& epi, int* flag_dev, cudaStream_t s) {
-  using Cfg = GntCfg<NOBJ, PAIR, SC_, SP>;
+  using Cfg = GntCfg<NOBJ, PAIR>;
   const int n_scenes = epi.M / NOBJ;
   const int cs = p->cluster;
   const int total = ((n_scenes + Cfg::SC - 1) / Cfg::SC) * (epi.N / BM / cs);      // work units per cluster
@@ -1783,7 +1568,7 @@ static int launch_gnt(const TcGemmPlan* p, const TcEpi& epi, int* flag_dev, cuda
   cfg.stream = s;
   cudaLaunchAttribute attr[2];
   int na = 0;
-  const bool pdl = tc_pdl_enabled(epi.M);
+  const bool pdl = pdl_enabled(epi.M);
   if (pdl) {
     attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[na].val.programmaticStreamSerializationAllowed = 1;
@@ -1802,14 +1587,14 @@ static int launch_gnt(const TcGemmPlan* p, const TcEpi& epi, int* flag_dev, cuda
       cfg.numAttrs = na;
       cfg.gridDim = dim3(max_cl * cs);
       int n = 0;
-      cached = (cudaOccupancyMaxActiveClusters(&n, k_gemm_gnt<NOBJ, PAIR, SC_, SP, TWO>, &cfg) == cudaSuccess && n > 0) ? n : max_cl;
+      cached = (cudaOccupancyMaxActiveClusters(&n, k_gemm_gnt<NOBJ, PAIR, TWO>, &cfg) == cudaSuccess && n > 0) ? n : max_cl;
     }
     if (cached < max_cl) max_cl = cached;
   }
   cfg.attrs = na ? attr : nullptr;
   cfg.numAttrs = na;
   cfg.gridDim = dim3((total < max_cl ? total : max_cl) * cs);
-  return (int)cudaLaunchKernelEx(&cfg, k_gemm_gnt<NOBJ, PAIR, SC_, SP, TWO>, p->tm_w, p->tm_a0, p->tm_a1, epi, flag_dev);
+  return (int)cudaLaunchKernelEx(&cfg, k_gemm_gnt<NOBJ, PAIR, TWO>, p->tm_w, p->tm_a0, p->tm_a1, epi, flag_dev);
 }
 
 int launch_gemm_tc(const TcGemmPlan* p, int M, cudaStream_t s) {
@@ -1818,24 +1603,14 @@ int launch_gemm_tc(const TcGemmPlan* p, int M, cudaStream_t s) {
   if (p->gnt) {
     int* fd = nullptr;
     cudaHostGetDevicePointer((void**)&fd, g_err_flag, 0);
-    // GroupNorm statistics exchange: 0 two CTA-wide barriers, 1 (default) warp-pair local (named 64-thread barriers).
-    // A/B on one box: no difference while the MMA issue was the slow side (profiles/round2_gnt_ab.txt: 39.3 / 43.2 / 66.3
+    // GroupNorm statistics exchange: warp-pair local (PAIR, named 64-thread barriers) rather than two CTA-wide
+    // barriers.  No difference while the MMA issue was the slow side (profiles/round2_gnt_ab.txt: 39.3 / 43.2 / 66.3
     // us vs 40.0 / 43.2 / 66.0 us); with the warp-uniform issue the residual blocks gain (41.5 -> 40.1 us) and the
-    // whole sample 1.1 % (900.5 -> 910.8 scenes/s, profiles/round2_probe_l2pf.txt)
-    static const int pair = getenv("DS_GNT_PAIR") ? atoi(getenv("DS_GNT_PAIR")) : 1;
-    if (epi.two_cta && p->cluster == 2) {
-      // A/B: the epilogue variants combined with the CTA pair (N = 12 only)
-      static const int spill2 = getenv("DS_GNT_SPILL") ? atoi(getenv("DS_GNT_SPILL")) : 0;
-      if (epi.n_obj == 12 && spill2) return launch_gnt<12, false, 0, true, true>(p, epi, fd, s);
-      if (epi.n_obj == 12 && pair) return launch_gnt<12, true, 0, false, true>(p, epi, fd, s);
-      return epi.n_obj == 21 ? launch_gnt<21, false, 0, false, true>(p, epi, fd, s) : launch_gnt<12, false, 0, false, true>(p, epi, fd, s);
-    }
-    if (epi.n_obj == 12 && gnt_scenes_per_tile(12) == 20) return launch_gnt<12, false, 20>(p, epi, fd, s);
-    // DS_GNT_SPILL=1 (A/B switch, N = 12): single TMEM read, normalisation pass from shared memory
-    static const int spill = getenv("DS_GNT_SPILL") ? atoi(getenv("DS_GNT_SPILL")) : 0;
-    if (spill && epi.n_obj == 12) return launch_gnt<12, false, 0, true>(p, epi, fd, s);
-    if (pair) return epi.n_obj == 21 ? launch_gnt<21, true>(p, epi, fd, s) : launch_gnt<12, true>(p, epi, fd, s);
-    return epi.n_obj == 21 ? launch_gnt<21, false>(p, epi, fd, s) : launch_gnt<12, false>(p, epi, fd, s);
+    // whole sample 1.1 % (900.5 -> 910.8 scenes/s, profiles/round2_probe_l2pf.txt).  The N = 21 CTA pair keeps the
+    // CTA-wide barriers.
+    if (p->cluster == 2)
+      return epi.n_obj == 21 ? launch_gnt<21, false, true>(p, epi, fd, s) : launch_gnt<12, true, true>(p, epi, fd, s);
+    return epi.n_obj == 21 ? launch_gnt<21, true>(p, epi, fd, s) : launch_gnt<12, true>(p, epi, fd, s);
   }
   const int num_m = (M + epi.tile_rows - 1) / epi.tile_rows;
   const int total_ct = ((num_m + p->cluster - 1) / p->cluster) * (epi.N / p->bn) * (epi.ksplit > 1 ? epi.ksplit : 1);
@@ -1843,7 +1618,7 @@ int launch_gemm_tc(const TcGemmPlan* p, int M, cudaStream_t s) {
   int* flag_dev = nullptr;
   cudaHostGetDevicePointer((void**)&flag_dev, g_err_flag, 0);
   if (p->gn) return launch_one<256, true>(p, epi, total_ct, flag_dev, s);
-  if (p->bn == 256 && epi.two_cta && p->cluster == 2) return launch_one<256, false, true>(p, epi, total_ct, flag_dev, s);
+  if (p->cluster == 2) return launch_one<256, false, true>(p, epi, total_ct, flag_dev, s);
   if (p->bn == 256) return launch_one<256, false>(p, epi, total_ct, flag_dev, s);
   return launch_one<128, false>(p, epi, total_ct, flag_dev, s);
 }

@@ -128,13 +128,11 @@ TcGemmPlan* tc_plan_create(const GemmArgs& g, int rows_capacity, char* err, int 
 void tc_plan_destroy(TcGemmPlan* p);
 void tc_plan_set_film(TcGemmPlan* p, const FilmRef& f);
 void tc_plan_set_trace(TcGemmPlan* p, unsigned long long* trace);
-// Programmatic-dependent-launch policy shared by every launcher of the library (pointwise.cu).  kind 0: tcgen05 GEMM
-// kernels (DS_TC_PDL), kind 1: pointwise kernels (DS_PW_PDL); values 0 off, 1 on, 2 (default) automatic: on when `rows`
-// (tokens of the launch) <= DS_PDL_ROWS (default 32768).  Measured on B200 (profiles/round2_probe_pdl.txt,
-// round2_probe_epi.txt), bedroom N = 12: 1 / 128 / 512 / 1024 / 2048 scenes per GPU gain 8 / 7.5 / 8 / 6 / 3 % (the ~5 us
-// kernel prologue is a large share of each launch), 4096 scenes lose 1.4 % (the chip runs at its power cap there and the
-// early-resident CTAs cost clock).
-bool pdl_enabled(int kind, int64_t rows);
+// Programmatic-dependent-launch policy shared by every launcher of the library (pointwise.cu): on when `rows` (tokens
+// of the launch) <= 32768.  Measured on B200 (profiles/round2_probe_pdl.txt, round2_probe_epi.txt), bedroom N = 12:
+// 1 / 128 / 512 / 1024 / 2048 scenes per GPU gain 8 / 7.5 / 8 / 6 / 3 % (the ~5 us kernel prologue is a large share of
+// each launch), 4096 scenes lose 1.4 % (the chip runs at its power cap there and the early-resident CTAs cost clock).
+bool pdl_enabled(int64_t rows);
 void tc_plan_set_atomic_out(TcGemmPlan* p, float* d32, int ldd, int ksplit);      // split-K, fp32 atomics (dW GEMMs)
 int tc_plan_tiles(const TcGemmPlan* p, int M);
 void tc_plan_set_residual(TcGemmPlan* p, const void* res);      // nullptr: plain store; == output: accumulate in place

@@ -7,29 +7,20 @@
 // LinearAttention :208-235, Attention :237-259, LinearAttentionCross :261-297) and
 // scene_synthesis/networks/diffusion_ddpm.py (q_sample :276-286, p_sample :339-352, p_losses :520-652).
 #include "kernels.cuh"
-#include <cstdlib>
 #include <utility>
 
 namespace ds {
-
-static constexpr int PDL_DEFAULT_MODE = 2;      // 0 off / 1 on / 2 automatic by launch size (see kernels.cuh)
 
 // Programmatic dependent launch for the pointwise kernels of the step program: launched with the PDL attribute, a
 // kernel may be scheduled while the previous kernel in the stream (a GEMM that issued griddepcontrol.launch_dependents)
 // drains; it touches no memory before `pdl_wait()`.  These kernels do NOT trigger their own dependents early (their
 // dependents are 96-register, 216 KB GEMM CTAs that would crowd out the remaining waves).
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-bool pdl_enabled(int kind, int64_t rows) {
-  static const int mode[2] = {getenv("DS_TC_PDL") ? atoi(getenv("DS_TC_PDL")) : PDL_DEFAULT_MODE,
-                              getenv("DS_PW_PDL") ? atoi(getenv("DS_PW_PDL")) : PDL_DEFAULT_MODE};
-  static const int64_t auto_rows = getenv("DS_PDL_ROWS") ? atoll(getenv("DS_PDL_ROWS")) : 32768;
-  const int m = mode[kind != 0];
-  return m == 2 ? rows <= auto_rows : m != 0;
-}
-// rows: tokens the launch works on (the automatic policy keys on it); the pointwise kernels pass their row count
+bool pdl_enabled(int64_t rows) { return rows <= 32768; }
+// rows: tokens the launch works on (the PDL policy keys on it); the pointwise kernels pass their row count
 template <typename... KArgs, typename... Args>
 static void launch_pdl_rows(int64_t rows, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args&&... args) {
-  const bool pdl = pdl_enabled(1, rows);
+  const bool pdl = pdl_enabled(rows);
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
@@ -662,8 +653,7 @@ template <typename T>
 void launch_linattn(const T* qkv, int ld, T* out, int ld_out, int n_scenes, int n_obj, cudaStream_t s) {
   if constexpr (sizeof(T) == 2) {       // bf16 mode: warp-level tensor-core variants
     const bool vec_ok = (ld % 8 == 0) && (ld_out % 2 == 0) && ((uintptr_t)qkv % 16 == 0) && ((uintptr_t)out % 4 == 0);
-    static const bool use_frag = !(getenv("DS_LINATTN_FRAG") && atoi(getenv("DS_LINATTN_FRAG")) == 0);
-    if (vec_ok && use_frag && n_obj <= 32) {
+    if (vec_ok && n_obj <= 32) {
       if (n_obj == 12) launch_pdl(k_linattn_frag<16, 12>, dim3(n_scenes), dim3(128), 0, s, qkv, ld, out, ld_out, n_scenes, n_obj);
       else if (n_obj == 21) launch_pdl(k_linattn_frag<32, 21>, dim3(n_scenes), dim3(128), 0, s, qkv, ld, out, ld_out, n_scenes, n_obj);
       else if (n_obj <= 16) launch_pdl(k_linattn_frag<16, 0>, dim3(n_scenes), dim3(128), 0, s, qkv, ld, out, ld_out, n_scenes, n_obj);
@@ -853,8 +843,7 @@ template <typename T>
 void launch_softattn(const T* qkv, int ld, T* out, int ld_out, int n_scenes, int n_obj, cudaStream_t s) {
   if constexpr (sizeof(T) == 2) {
     const bool vec_ok = (ld % 8 == 0) && (ld_out % 2 == 0) && ((uintptr_t)qkv % 16 == 0) && ((uintptr_t)out % 4 == 0);
-    static const bool use_frag = !(getenv("DS_SOFTATTN_FRAG") && atoi(getenv("DS_SOFTATTN_FRAG")) == 0);
-    if (vec_ok && use_frag && n_obj <= 32) {
+    if (vec_ok && n_obj <= 32) {
       if (n_obj == 12) launch_pdl(k_softattn_frag<16, 12>, dim3(n_scenes), dim3(128), 0, s, qkv, ld, out, ld_out, n_scenes, n_obj);
       else if (n_obj == 21) launch_pdl(k_softattn_frag<32, 21>, dim3(n_scenes), dim3(128), 0, s, qkv, ld, out, ld_out, n_scenes, n_obj);
       else if (n_obj <= 16) launch_pdl(k_softattn_frag<16, 0>, dim3(n_scenes), dim3(128), 0, s, qkv, ld, out, ld_out, n_scenes, n_obj);

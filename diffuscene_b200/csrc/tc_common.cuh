@@ -5,9 +5,6 @@
 #include <cuda_bf16.h>
 #include <stdint.h>
 
-#include <cstdlib>
-#include <type_traits>
-
 #include "kernels.cuh"
 
 namespace ds {
@@ -21,9 +18,6 @@ __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)_
 
 __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
@@ -58,29 +52,6 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, int* er
   }
 }
 
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-      ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar,
-                                               uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%2, %3}], [%4], %5;"
-      ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar), "h"(cta_mask)
-      : "memory");
-}
-__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, int c0, int c1, uint32_t src) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%1, %2}], [%3];"
-               ::"l"(map), "r"(c0), "r"(c1), "r"(src)
-               : "memory");
-  asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-}
-__device__ __forceinline__ void tma_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void tma_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -112,39 +83,6 @@ __host__ __device__ constexpr uint64_t umma_desc_hi_sw128() {
 __device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr, uint64_t hi) {
   return hi | (uint64_t)((smem_addr & 0x3FFFFu) >> 4);   // start address in 16-byte units
 }
-// D(tmem, fp32) (+)= A(smem, bf16) * B(smem, bf16)^T, M = 128, N from the instruction descriptor, K = 16
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                          uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t cta_mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(bar), "h"(cta_mask)
-      : "memory");
-}
-// ---- warp-uniform issue (UNI = true) ----------------------------------------------------------------------------
-// The single-thread roles (TMA producer, MMA issuer) can run their loops with the WHOLE warp active: control flow is
-// then warp-uniform, descriptors / barrier addresses / loop counters live in uniform registers, and one elected lane
-// executes each tcgen05 / TMA instruction.  Inside an `if (lane == 0)` region the compiler cannot prove that a single
-// thread is active and wraps every UTCHMMA / UTCBAR / UTMALDG in an ELECT + 5 x R2UR.BROADCAST + BRA.U.ANY waterfall
-// (19 SASS instructions per MMA on the issuing thread; 4 MMAs + commit back to back in the uniform form).  The warp
-// index must be taken through uniform_warp_idx() for this.  elect.sync picks the same lane for the same member mask
-// every time, so the commits track that lane's MMAs.  UNI = false keeps the lane-0 form (A/B switch DS_TC_UNI).
-// host side: the A/B switch shared by every tcgen05 kernel of the library (default: uniform issue)
-inline int tc_uniform_issue() {
-  static const int v = getenv("DS_TC_UNI") ? atoi(getenv("DS_TC_UNI")) : 1;
-  return v;
-}
-inline bool tc_pdl_enabled(int rows) { return pdl_enabled(0, rows); }      // policy: kernels.cuh
 // launch with the optional programmatic-stream-serialization attribute
 template <typename... KArgs, typename... Args>
 inline int tc_launch(void (*kern)(KArgs...), int grid, int threads, size_t smem, cudaStream_t s, bool pdl, Args&&... args) {
@@ -162,101 +100,49 @@ inline int tc_launch(void (*kern)(KArgs...), int grid, int threads, size_t smem,
   }
   return (int)cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
 }
+// ---- warp-uniform issue --------------------------------------------------------------------------------------------
+// The single-thread roles (TMA producer, MMA issuer) run their loops with the WHOLE warp active: control flow is
+// warp-uniform, descriptors / barrier addresses / loop counters live in uniform registers, and one elected lane
+// executes each tcgen05 / TMA instruction.  Inside an `if (lane == 0)` region the compiler cannot prove that a single
+// thread is active and wraps every UTCHMMA / UTCBAR / UTMALDG in an ELECT + 5 x R2UR.BROADCAST + BRA.U.ANY waterfall
+// (19 SASS instructions per MMA on the issuing thread; 4 MMAs + commit back to back in the uniform form).  The warp
+// index must be taken through uniform_warp_idx() for this.  elect.sync picks the same lane for the same member mask
+// every time, so the commits track that lane's MMAs.
 __device__ __forceinline__ int uniform_warp_idx() { return __shfl_sync(0xffffffffu, int(threadIdx.x >> 5), 0); }
 
-template <bool UNI>
-__device__ __forceinline__ void umma_issue(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                           uint32_t accumulate) {
-  if constexpr (UNI) {
-    asm volatile(
-        "{\n\t.reg .pred p, e;\n\t"
-        "elect.sync _|e, 0xffffffff;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "@e tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-  } else {
-    umma_bf16(d_tmem, a_desc, b_desc, idesc, accumulate);
-  }
+// D(tmem, fp32) (+)= A(smem, bf16) * B(smem, bf16)^T, M = 128, N from the instruction descriptor, K = 16
+__device__ __forceinline__ void umma_issue_elect(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
+                                                 uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p, e;\n\t"
+      "elect.sync _|e, 0xffffffff;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "@e tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+      : "memory");
 }
-template <bool UNI>
-__device__ __forceinline__ void umma_arrive(uint32_t bar) {
-  if constexpr (UNI) {
-    asm volatile(
-        "{\n\t.reg .pred e;\n\t"
-        "elect.sync _|e, 0xffffffff;\n\t"
-        "@e tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n\t}" ::"r"(bar)
-        : "memory");
-  } else {
-    umma_commit(bar);
-  }
+// completion of the MMAs issued so far -> one arrival on `bar`
+__device__ __forceinline__ void umma_arrive_elect(uint32_t bar) {
+  asm volatile(
+      "{\n\t.reg .pred e;\n\t"
+      "elect.sync _|e, 0xffffffff;\n\t"
+      "@e tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];\n\t}" ::"r"(bar)
+      : "memory");
 }
-template <bool UNI>
-__device__ __forceinline__ void umma_arrive_mc(uint32_t bar, uint16_t cta_mask) {
-  if constexpr (UNI) {
-    asm volatile(
-        "{\n\t.reg .pred e;\n\t"
-        "elect.sync _|e, 0xffffffff;\n\t"
-        "@e tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;\n\t}"
-        ::"r"(bar), "h"(cta_mask)
-        : "memory");
-  } else {
-    umma_commit_mc(bar, cta_mask);
-  }
+__device__ __forceinline__ void mbar_expect_tx_elect(uint32_t bar, uint32_t bytes) {
+  asm volatile(
+      "{\n\t.reg .pred e;\n\t"
+      "elect.sync _|e, 0xffffffff;\n\t"
+      "@e mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n\t}" ::"r"(bar), "r"(bytes)
+      : "memory");
 }
-template <bool UNI>
-__device__ __forceinline__ void mbar_expect_tx_r(uint32_t bar, uint32_t bytes) {
-  if constexpr (UNI) {
-    asm volatile(
-        "{\n\t.reg .pred e;\n\t"
-        "elect.sync _|e, 0xffffffff;\n\t"
-        "@e mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n\t}" ::"r"(bar), "r"(bytes)
-        : "memory");
-  } else {
-    mbar_expect_tx(bar, bytes);
-  }
-}
-template <bool UNI>
-__device__ __forceinline__ void tma_load_2d_r(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-  if constexpr (UNI) {
-    asm volatile(
-        "{\n\t.reg .pred e;\n\t"
-        "elect.sync _|e, 0xffffffff;\n\t"
-        "@e cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];\n\t}"
-        ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar)
-        : "memory");
-  } else {
-    tma_load_2d(dst, map, c0, c1, bar);
-  }
-}
-template <bool UNI>
-__device__ __forceinline__ void tma_load_2d_mc_r(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar,
-                                                 uint16_t cta_mask) {
-  if constexpr (UNI) {
-    asm volatile(
-        "{\n\t.reg .pred e;\n\t"
-        "elect.sync _|e, 0xffffffff;\n\t"
-        "@e cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-        " [%0], [%1, {%2, %3}], [%4], %5;\n\t}"
-        ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar), "h"(cta_mask)
-        : "memory");
-  } else {
-    tma_load_2d_mc(dst, map, c0, c1, bar, cta_mask);
-  }
-}
-
-// L2 prefetch of a tile a TMA load will fetch later (no shared-memory destination, no barrier)
-template <bool UNI>
-__device__ __forceinline__ void tma_prefetch_2d_r(const CUtensorMap* map, int c0, int c1) {
-  if constexpr (UNI) {
-    asm volatile(
-        "{\n\t.reg .pred e;\n\t"
-        "elect.sync _|e, 0xffffffff;\n\t"
-        "@e cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];\n\t}" ::"l"(map), "r"(c0), "r"(c1)
-        : "memory");
-  } else {
-    asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(map), "r"(c0), "r"(c1) : "memory");
-  }
+__device__ __forceinline__ void tma_load_2d_elect(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
+  asm volatile(
+      "{\n\t.reg .pred e;\n\t"
+      "elect.sync _|e, 0xffffffff;\n\t"
+      "@e cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];\n\t}"
+      ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar)
+      : "memory");
 }
 
 // ---- CTA pair (cta_group::2): one UMMA of M = 256 spans the two SMs of a cluster of 2 ------------------------------

@@ -233,7 +233,6 @@ static int train_init(ds_handle* h) {
   CK(cudaMalloc(&t->warena, total));
   CK(cudaMemset(t->warena, 0, total));
   t->use_tc = h->use_tc;
-  if (const char* e = getenv("DS_TRAIN_TC")) t->use_tc = t->use_tc && atoi(e) != 0;
   if (t->use_tc) {
     CK(cudaMalloc(&t->wtarena, total));
     CK(cudaMemset(t->wtarena, 0, total));

@@ -52,79 +52,6 @@ run_task() {
         bench.py --gpus 2 --config train --steps 5 --warmup 3 2>gpurun_out/${TAG}_dp2_train.err | tail -1 | tee gpurun_out/${TAG}_dp2_train.json
       timeout 600 python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29513 \
         bench.py --gpus 2 --steps 2 --warmup 2 --no-cpu-baseline "$@" 2>gpurun_out/${TAG}_dp2_sample.err | tail -1 | tee gpurun_out/${TAG}_dp2_sample.json ;;
-    probe-wide)    # A/B of the wide TMEM loads in the statistics pass of k_gemm_gnt
-      for w in 0 1 0 1; do
-        echo "== DS_GNT_WIDE1=$w"
-        DS_GNT_WIDE1=$w GNT_ONLY=1 timeout 300 python tests/gpu_trace_gemm.py 2>&1 | grep -E "^(GNT|   check GNT)" | grep -E "M=49152|MISMATCH"
-      done | tee gpurun_out/${TAG}_probe_wide.txt ;;
-    probe-sc)      # A/B of the k_gemm_gnt tile width (16 vs 20 scenes) with numeric checks, then a short bench of each
-      for sc in 16 20; do
-        echo "== DS_GNT_SC=$sc"
-        DS_GNT_SC=$sc GNT_ONLY=1 timeout 300 python tests/gpu_trace_gemm.py 2>&1 | grep -E "^(GNT|   check GNT|   prod_wait)" | grep -B0 -A1 -E "GNT.*M=49152|check GNT|MISMATCH" | grep -v "^--"
-      done | tee gpurun_out/${TAG}_probe_sc.txt
-      for sc in 16 20; do
-        DS_GNT_SC=$sc timeout 300 python bench.py --steps 2 --warmup 2 --no-cpu-baseline --no-e2e 2>/dev/null | python -c "import sys,json; d=json.loads(sys.stdin.read()); print('SC=$sc', d['value'], d['ms_per_step'], d['clocks'])"
-      done | tee -a gpurun_out/${TAG}_probe_sc.txt ;;
-    probe-spill)   # A/B of the single-TMEM-read epilogue (DS_GNT_SPILL) with numeric checks, then a short bench of each
-      for sp in 0 1; do
-        echo "== DS_GNT_SPILL=$sp"
-        DS_GNT_SPILL=$sp GNT_ONLY=1 timeout 300 python tests/gpu_trace_gemm.py 2>&1 | grep -E "^(GNT|   check GNT|   prod_wait)" | grep -B0 -A1 -E "GNT.*M=49152|check GNT|MISMATCH" | grep -v "^--"
-      done | tee gpurun_out/${TAG}_probe_spill.txt
-      for sp in 0 1; do
-        DS_GNT_SPILL=$sp timeout 300 python bench.py --steps 2 --warmup 2 --no-cpu-baseline --no-e2e 2>/dev/null | python -c "import sys,json; d=json.loads(sys.stdin.read()); print('SPILL=$sp', d['value'], d['ms_per_step'], d['parity_max_abs'], d['clocks'])"
-      done | tee -a gpurun_out/${TAG}_probe_spill.txt ;;
-    probe-ab)      # A/B of the k_gemm_gnt switches on one box: statistics exchange x residual L2 prefetch
-      for pair in 0 1; do for pf in 0 1; do
-        echo "== DS_GNT_PAIR=$pair DS_GNT_PREFETCH=$pf"
-        DS_GNT_PAIR=$pair DS_GNT_PREFETCH=$pf GNT_ONLY=1 timeout 300 python tests/gpu_trace_gemm.py 2>&1 | grep -E "^(GNT|T qkv|T to_out|T enc.l1)" | grep "M=49152"
-      done; done | tee gpurun_out/${TAG}_probe_ab.txt ;;
-    probe-uni)     # A/B of the warp-uniform issue (DS_TC_UNI) and the CTA-pair policy (DS_GNT_2CTA) with numeric checks, then short benches
-      for cfg in "DS_TC_UNI=0 DS_GNT_2CTA=0" "DS_TC_UNI=1 DS_GNT_2CTA=0" "DS_TC_UNI=1 DS_GNT_2CTA=2" "DS_TC_UNI=1 DS_GNT_2CTA=1"; do
-        echo "== $cfg"
-        env $cfg GNT_ONLY=1 timeout 300 python tests/gpu_trace_gemm.py 2>&1 | grep -A1 -E "M=49152|MISMATCH|FAILED" | grep -v "^--" | cut -c1-220
-      done | tee gpurun_out/${TAG}_probe_uni.txt
-      for cfg in "DS_TC_UNI=0 DS_GNT_2CTA=0" "DS_TC_UNI=1 DS_GNT_2CTA=0" "DS_TC_UNI=1 DS_GNT_2CTA=2" "DS_TC_UNI=1 DS_GNT_2CTA=1"; do
-        env $cfg timeout 300 python bench.py --steps 2 --warmup 2 --no-cpu-baseline --no-e2e 2>gpurun_out/${TAG}_bench_ab.err | tail -1 | python -c "import sys,json; d=json.loads(sys.stdin.read()); print('$cfg', d['value'], d['ms_per_step'], d['parity_max_abs'], d['clocks'])" || tail -5 gpurun_out/${TAG}_bench_ab.err
-      done 2>&1 | tee -a gpurun_out/${TAG}_probe_uni.txt ;;
-    probe-pdl)     # programmatic dependent launch at small per-GPU batches (latency / strong-scaling points)
-      for cfg in "DS_TC_PDL=0 DS_PW_PDL=0" "DS_TC_PDL=1 DS_PW_PDL=1"; do
-        for b in "--config lat1" "--batch 128" "--batch 512" "--batch 1024"; do
-          env $cfg timeout 300 python bench.py $b --steps 2 --warmup 2 --no-cpu-baseline --no-e2e 2>&1 | tail -1 | python -c "import sys,json; d=json.loads(sys.stdin.read()); print('$cfg', '$b', d['value'], d['ms_per_step'], d.get('parity_max_abs'), d['clocks']['sm_mhz'])"
-        done
-      done 2>&1 | tee gpurun_out/${TAG}_probe_pdl.txt ;;
-    probe-epi)     # epilogue variants of k_gemm_gnt again, now that the MMA side is fast (uniform issue): probe + short benches
-      for cfg in "DS_GNT_SPILL=0" "DS_GNT_SPILL=1" "DS_GNT_SC=20" "DS_GNT_PAIR=1"; do
-        echo "== $cfg"
-        env $cfg GNT_ONLY=1 timeout 300 python tests/gpu_trace_gemm.py 2>&1 | grep -A1 -E "^GNT.*M=49152|MISMATCH|FAILED" | grep -v "^--" | cut -c1-220
-      done | tee gpurun_out/${TAG}_probe_epi.txt
-      for cfg in "DS_TC_UNI=1" "DS_TC_UNI=0 DS_GNT_2CTA=0" "DS_GNT_SPILL=1" "DS_GNT_SC=20" "DS_TC_PDL=1 DS_PW_PDL=1" "DS_TC_PDL=1 DS_PW_PDL=1 BATCH=2048" "BATCH=2048"; do
-        b=4096; case "$cfg" in *BATCH=2048*) b=2048;; esac
-        env $cfg timeout 300 python bench.py --batch $b --steps 2 --warmup 2 --no-cpu-baseline --no-e2e 2>gpurun_out/${TAG}_bench_ab.err | tail -1 | python -c "import sys,json; d=json.loads(sys.stdin.read()); print('$cfg', d['value'], d['ms_per_step'], d.get('parity_max_abs'), d['clocks'])" || tail -5 gpurun_out/${TAG}_bench_ab.err
-      done 2>&1 | tee -a gpurun_out/${TAG}_probe_epi.txt ;;
-    probe-l2pf)    # L2 prefetch of the next activation tile (DS_TC_L2PF), pair-local statistics again; short benches
-      for cfg in "DS_TC_L2PF=0" "DS_TC_L2PF=1"; do
-        echo "== $cfg"
-        env $cfg GNT_ONLY=1 timeout 300 python tests/gpu_trace_gemm.py 2>&1 | grep -A1 -E "M=49152|MISMATCH|FAILED" | grep -v "^--\|^   prod" | cut -c1-220
-      done | tee gpurun_out/${TAG}_probe_l2pf.txt
-      for cfg in "DS_TC_L2PF=1" "DS_GNT_PAIR=1" "DS_TC_L2PF=1 DS_GNT_PAIR=1" "DS_TC_L2PF=0"; do
-        env $cfg timeout 300 python bench.py --steps 2 --warmup 2 --no-cpu-baseline --no-e2e 2>gpurun_out/${TAG}_bench_ab.err | tail -1 | python -c "import sys,json; d=json.loads(sys.stdin.read()); print('$cfg', d['value'], d['ms_per_step'], d.get('parity_max_abs'), d['clocks'])" || tail -5 gpurun_out/${TAG}_bench_ab.err
-      done 2>&1 | tee -a gpurun_out/${TAG}_probe_l2pf.txt ;;
-    probe-pairepi) # CTA pair everywhere combined with the epilogue variants (single TMEM read / pair-local statistics)
-      for cfg in "DS_GNT_2CTA=1 DS_GNT_SPILL=1" "DS_GNT_2CTA=1 DS_GNT_PAIR=1"; do
-        echo "== $cfg"
-        env $cfg GNT_ONLY=1 timeout 300 python tests/gpu_trace_gemm.py 2>&1 | grep -A1 -E "^GNT.*M=49152|check GNT|MISMATCH|FAILED" | grep -v "^--" | cut -c1-220
-      done | tee gpurun_out/${TAG}_probe_pairepi.txt
-      for cfg in "DS_GNT_2CTA=1 DS_GNT_SPILL=1" "DS_GNT_2CTA=1 DS_GNT_PAIR=1"; do
-        env $cfg timeout 300 python bench.py --steps 2 --warmup 2 --no-cpu-baseline --no-e2e 2>gpurun_out/${TAG}_bench_ab.err | tail -1 | python -c "import sys,json; d=json.loads(sys.stdin.read()); print('$cfg', d['value'], d['ms_per_step'], d.get('parity_max_abs'), d['clocks'])" || tail -5 gpurun_out/${TAG}_bench_ab.err
-      done 2>&1 | tee -a gpurun_out/${TAG}_probe_pairepi.txt ;;
-    probe-tc2)     # CTA-pair variant of the row-major kernel k_gemm_tc (DS_TC_2CTA): numeric checks + timings, short benches
-      for cfg in "DS_TC_2CTA=0" "DS_TC_2CTA=1"; do
-        echo "== $cfg"
-        env $cfg PLAIN_ONLY=1 timeout 300 python tests/gpu_trace_gemm.py 2>&1 | grep -E "check|M=49152|MISMATCH|FAILED|rror|mma_wait" | grep -v "OK$" | cut -c1-220
-      done | tee gpurun_out/${TAG}_probe_tc2.txt
-      for cfg in "DS_TC_2CTA=1" "DS_TC_2CTA=0"; do
-        env $cfg timeout 300 python bench.py --steps 2 --warmup 2 --no-e2e --no-cpu-baseline 2>gpurun_out/${TAG}_bench_ab.err | tail -1 | python -c "import sys,json; d=json.loads(sys.stdin.read()); print('$cfg', d['value'], d['ms_per_step'], d.get('parity_max_abs'), d.get('parity_class_argmax_agreement'), d['clocks'])" || tail -5 gpurun_out/${TAG}_bench_ab.err
-      done 2>&1 | tee -a gpurun_out/${TAG}_probe_tc2.txt ;;
     py)
       timeout 900 python "$@" 2>&1 | tail -40 | tee gpurun_out/${TAG}_py.log ;;
     *) echo "unknown task $task"; return 2 ;;

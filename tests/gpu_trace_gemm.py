@@ -76,8 +76,6 @@ def run(M, N, K, n_obj=0, res=False, tag="", gnt=False, check=False, plain_act=N
     print("   " + "  ".join("%s=%.0f" % (n, t[:, i].mean()) for i, n in enumerate(names)))
 
 
-cl = os.environ.get("DS_TC_CLUSTER", "1")
-print("cluster size", cl)
 M = 49152
 if os.environ.get("PLAIN_ONLY"):      # row-major plain kernel (k_gemm_tc): numeric checks incl. odd tile counts, then timings
     for m_chk in (128 * 5, 128 * 5 - 37, 12 * 1000, 128 * 301):
