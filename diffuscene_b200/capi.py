@@ -80,6 +80,7 @@ def load(rebuild: bool = False):
         "ds_train_param_count": (C.c_int64, [H]),
         "ds_train_step": (C.c_int, [H, p, p, p, p, p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, p, C.c_float, p, p, p, p,
                                     C.c_int32, p]),
+        "ds_train_set_context_cross": (C.c_int, [H, p, C.c_int32, C.c_int32, p]),
         "ds_train_set_buckets": (C.c_int, [H, p, C.c_int32, p]),
         "ds_train_phase_ms": (C.c_int, [H, p]),
         "ds_sumsq": (C.c_int, [p, C.c_int64, p, p]),
@@ -109,7 +110,7 @@ EXPORTED = ["ds_create", "ds_destroy", "ds_last_error", "ds_version", "ds_load_w
             "ds_expected_weight_count", "ds_expected_weight", "ds_set_schedule", "ds_set_context",
             "ds_set_context_cross", "ds_denoise_forward", "ds_denoise_forward_host", "ds_sample_loop",
             "ds_sample_loop_host", "ds_traj_count", "ds_p_sample_step", "ds_q_sample", "ds_p_losses", "ds_retrieve_objects",
-            "ds_train_param_count", "ds_train_step", "ds_train_set_buckets", "ds_train_phase_ms", "ds_sumsq", "ds_adam_step",
+            "ds_train_param_count", "ds_train_step", "ds_train_set_context_cross", "ds_train_set_buckets", "ds_train_phase_ms", "ds_sumsq", "ds_adam_step",
             "ds_plan_describe", "ds_plan_export_json", "ds_enable_taps", "ds_read_tap", "ds_launch_count", "ds_graph_build_count", "ds_gnt_weight_row", "ds_profile_ops",
             "ds_test_gemm_bf16", "ds_test_gemm_trace"]
 

@@ -7,6 +7,7 @@
 //   Block           k_gn_bwd: GroupNorm(8) + affine + FiLM + SiLU (+ residual passthrough) in one pass per (scene, group)
 //   LayerNorm       k_ln_bwd
 //   LinearAttention k_linattn_bwd, Attention k_softattn_bwd (one warp per (scene, head), everything in shared memory)
+//   LinearAttentionCross k_xattn_bwd (one CTA per scene, one warp per head; text tokens streamed in chunks)
 //   loss            k_p_losses_bwd: d(loss)/d(model output) for the MSE terms and the IoU regulariser
 //   weights         k_ws_unpack: packed-matrix gradients -> named tensors through the weight-standardisation adjoint
 //   optimizer       k_adam, k_sumsq (global gradient norm for clip_grad_norm_)
@@ -651,6 +652,100 @@ void launch_linattn_bwd(const T* qkv, int ld, const T* dout, int ldo, T* dqkv, i
   if (n_scenes > 0) k_linattn_bwd<T><<<n_scenes * 4, 32, 0, s>>>(qkv, ld, dout, ldo, dqkv, lddq, n_scenes, N);
 }
 
+// LinearAttentionCross core (denoise_net.py:261-297): q^ = softmax over the 32 head channels * 32^-1/2 (per object),
+// k^ = softmax over the L text tokens, ctx[d][e] = sum_l k^[l][d] v[l][e], out[n][e] = sum_d ctx[d][e] q^[n][d].
+// One CTA per scene, one warp per head.  q^, k^ and ctx are recomputed from q and the layer's k | v; the text tokens
+// are streamed in chunks of XATTN_CHUNK, so shared memory is fixed for every L.  Writes dq (overwrites, or adds when
+// dq_accumulate) and d(k | v) of the layer: dctx[d][e] = sum_n q^[n][d] dout[n][e], dv[l][e] = sum_d k^[l][d] dctx[d][e],
+// dk^[l][d] = sum_e dctx[d][e] v[l][e], dk = k^ (dk^ - sum_l dk^ k^).
+template <typename T>
+__global__ void __launch_bounds__(128) k_xattn_bwd(const T* __restrict__ q, int ldq, const T* __restrict__ dout, int ldo,
+                                                   const T* __restrict__ kv, int ld_kv, T* __restrict__ dq, int lddq,
+                                                   int dq_accumulate, T* __restrict__ dkv, int ld_dkv, int n_obj, int L) {
+  __shared__ float sm[4][2][XATTN_CHUNK][33];
+  const int lane = threadIdx.x & 31, h = threadIdx.x >> 5;
+  const int scene = blockIdx.x;
+  float (*A)[33] = sm[h][0];
+  float (*Bv)[33] = sm[h][1];
+  const T* kvs = kv + (int64_t)scene * L * ld_kv;
+  T* dkvs = dkv + (int64_t)scene * L * ld_dkv;
+  const float scale = 0.17677669529663687f;      // 32^-1/2
+  float kmax, kinv;
+  xattn_k_stats(kvs, ld_kv, L, h, lane, kmax, kinv);
+  float ctx[32];      // lane = d: ctx[e] = ctx[d][e]
+  xattn_context<T, true>(kvs, ld_kv, L, h, lane, kmax, kinv, A, Bv, ctx);
+  // object side (n_obj <= 32 rows): A = softmax(q) unscaled, Bv = dout; lane = channel
+  const int64_t row0 = (int64_t)scene * n_obj;
+  for (int n = 0; n < n_obj; ++n) {
+    const float v = ldf(q + (row0 + n) * ldq + h * 32 + lane);
+    const float e = expf(v - warp_max(v));
+    A[n][lane] = e / warp_sum(e);
+    Bv[n][lane] = ldf(dout + (row0 + n) * ldo + h * 32 + lane);
+  }
+  __syncwarp();
+  float dctx[32];      // lane = d
+#pragma unroll
+  for (int e = 0; e < 32; ++e) dctx[e] = 0.f;
+  for (int n = 0; n < n_obj; ++n) {
+    const float qs = A[n][lane];
+    float g = 0.f;
+#pragma unroll
+    for (int e = 0; e < 32; ++e) {
+      const float de = Bv[n][e];
+      dctx[e] = fmaf(qs * scale, de, dctx[e]);
+      g = fmaf(ctx[e], de, g);
+    }
+    g *= scale;      // gradient w.r.t. the softmaxed (unscaled) q
+    const float r = qs * (g - warp_sum(g * qs));
+    T* p = dq + (row0 + n) * lddq + h * 32 + lane;
+    stf(p, dq_accumulate ? ldf(p) + r : r);
+  }
+  __syncwarp();
+  // lane = e needs column e of dctx for dv: transpose through the first tile
+#pragma unroll
+  for (int e = 0; e < 32; ++e) A[lane][e] = dctx[e];
+  __syncwarp();
+  float dctxT[32];      // lane = e: dctxT[d] = dctx[d][e]
+#pragma unroll
+  for (int d = 0; d < 32; ++d) dctxT[d] = A[d][lane];
+  __syncwarp();
+  // pass 1 over the tokens: dv, and S[d] = sum_l dk^[l][d] k^[l][d]; pass 2: dk
+  float S = 0.f;
+  for (int pass = 0; pass < 2; ++pass) {
+    for (int l0 = 0; l0 < L; l0 += XATTN_CHUNK) {
+      const int nl = min(XATTN_CHUNK, L - l0);
+      for (int l = 0; l < nl; ++l) {
+        const T* p = kvs + (int64_t)(l0 + l) * ld_kv + h * 32 + lane;
+        A[l][lane] = expf(ldf(p) - kmax) * kinv;
+        Bv[l][lane] = ldf(p + 128);
+      }
+      __syncwarp();
+      for (int l = 0; l < nl; ++l) {
+        const float kd = A[l][lane];
+        float dkh = 0.f;
+#pragma unroll
+        for (int e = 0; e < 32; ++e) dkh = fmaf(dctx[e], Bv[l][e], dkh);
+        T* o = dkvs + (int64_t)(l0 + l) * ld_dkv + h * 32 + lane;
+        if (pass == 0) {
+          S = fmaf(dkh, kd, S);
+          float dv = 0.f;
+#pragma unroll
+          for (int d = 0; d < 32; ++d) dv = fmaf(A[l][d], dctxT[d], dv);
+          stf(o + 128, dv);
+        } else {
+          stf(o, kd * (dkh - S));
+        }
+      }
+      __syncwarp();
+    }
+  }
+}
+template <typename T>
+void launch_xattn_bwd(const T* q, int ldq, const T* dout, int ldo, const T* kv, int ld_kv, T* dq, int lddq, int dq_accumulate,
+                      T* dkv, int ld_dkv, int n_scenes, int n_obj, int L, cudaStream_t s) {
+  if (n_scenes > 0) k_xattn_bwd<T><<<n_scenes, 128, 0, s>>>(q, ldq, dout, ldo, kv, ld_kv, dq, lddq, dq_accumulate, dkv, ld_dkv, n_obj, L);
+}
+
 // Attention (denoise_net.py:237-259): sim[i][j] = scale * sum_d q[d][i] k[d][j], attn = softmax_j, out[i][d] = sum_j attn[i][j] v[j][d]
 template <typename T>
 __global__ void __launch_bounds__(32) k_softattn_bwd(const T* __restrict__ qkv, int ld, const T* __restrict__ dout, int ldo,
@@ -1026,6 +1121,8 @@ void launch_adam(float* p, const float* g, float* m, float* v, int64_t n, float 
                                  int, cudaStream_t);                                                                  \
   template void launch_linattn_bwd<T>(const T*, int, const T*, int, T*, int, int, int, cudaStream_t);                 \
   template void launch_softattn_bwd<T>(const T*, int, const T*, int, T*, int, int, int, cudaStream_t);                \
+  template void launch_xattn_bwd<T>(const T*, int, const T*, int, const T*, int, T*, int, int, T*, int, int, int, int, \
+                                    cudaStream_t);                                                                    \
   template void launch_p_losses_bwd<T>(const float*, const float*, const float*, const T*, int, const int64_t*,       \
                                        const float*, const float*, const float*, const float*, const float*,          \
                                        const float*, LossArgs, T*, int, int, int, float, cudaStream_t);               \

@@ -46,6 +46,44 @@ __device__ __forceinline__ float warp_max(float v) {
   return v;
 }
 
+// ---- cross linear attention, text side (LinearAttentionCross, denoise_net.py:261-297) ----
+// kv rows of one scene: [L][ld], k of head h at columns h*32 .. h*32+31, v at 128 + h*32 ..; one warp per head.
+// The L text tokens are streamed through two [XATTN_CHUNK][33] shared tiles per warp, so shared memory does not grow
+// with L (k_xattn_prepare, k_xattn_bwd).
+constexpr int XATTN_CHUNK = 32;
+// softmax over L of k channel d = lane: max and 1 / sum(exp(k - max)), summed in token order
+template <typename T>
+__device__ __forceinline__ void xattn_k_stats(const T* kv, int ld, int L, int h, int lane, float& kmax, float& kinv) {
+  float m = -INFINITY;
+  for (int l = 0; l < L; ++l) m = fmaxf(m, ldf(kv + (int64_t)l * ld + h * 32 + lane));
+  float s = 0.f;
+  for (int l = 0; l < L; ++l) s += expf(ldf(kv + (int64_t)l * ld + h * 32 + lane) - m);
+  kmax = m;
+  kinv = 1.0f / s;
+}
+// ctx[d][e] = sum_l softmax_L(k)[l][d] v[l][e].  LANE_D: lane = d, acc[e] = ctx[d][e]; otherwise lane = e, acc[d]
+template <typename T, bool LANE_D>
+__device__ __forceinline__ void xattn_context(const T* kv, int ld, int L, int h, int lane, float kmax, float kinv,
+                                              float (*Ks)[33], float (*Vs)[33], float* acc) {
+#pragma unroll
+  for (int i = 0; i < 32; ++i) acc[i] = 0.f;
+  for (int l0 = 0; l0 < L; l0 += XATTN_CHUNK) {
+    const int n = min(XATTN_CHUNK, L - l0);
+    for (int l = 0; l < n; ++l) {
+      const T* p = kv + (int64_t)(l0 + l) * ld + h * 32 + lane;
+      Ks[l][lane] = expf(ldf(p) - kmax) * kinv;
+      Vs[l][lane] = ldf(p + 128);
+    }
+    __syncwarp();
+    for (int l = 0; l < n; ++l) {
+      const float mine = LANE_D ? Ks[l][lane] : Vs[l][lane];
+#pragma unroll
+      for (int i = 0; i < 32; ++i) acc[i] = fmaf(LANE_D ? Vs[l][i] : Ks[l][i], mine, acc[i]);
+    }
+    __syncwarp();
+  }
+}
+
 // ---- Philox4x32-10 counter-based RNG (Salmon et al. 2011), one call -> 4 x u32 ----
 __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
   const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;

@@ -667,7 +667,8 @@ extern "C" int ds_set_context_cross(ds_handle* h, const float* cross_dev, int32_
     g.a0 = cross_dev; g.lda0 = TD; g.k0 = TD; g.w = h->kv_w[l]; g.ldw = TD; g.d = kv; g.ldd = 256;
     g.M = batch * L; g.N = 256; g.act = ACT_NONE;
     launch_gemm_f32(g, s);
-    launch_xattn_prepare(kv, 256, h->xctx + (size_t)l * batch * 4096, batch, L, s);
+    launch_xattn_prepare<float>(kv, 256, h->xctx + (size_t)l * batch * 4096, batch, L, s);
+    CK(cudaGetLastError());
     h->launches += 2;
   }
   CK(cudaFreeAsync(kv, s));

@@ -38,7 +38,9 @@ void launch_softattn(const T* qkv, int ld, T* out, int ld_out, int n_scenes, int
 template <typename T>
 void launch_xattn_apply(const T* q, int ldq, const float* ctx, T* out, int ld_out, int n_scenes, int n_obj,
                         cudaStream_t s);
-void launch_xattn_prepare(const float* kv, int ld_kv, float* ctx, int n_scenes, int L, cudaStream_t s);
+// kv: [n_scenes * L, ld_kv] rows of k | v (128 columns each) in storage type T; any 1 <= L <= 512
+template <typename T>
+void launch_xattn_prepare(const T* kv, int ld_kv, float* ctx, int n_scenes, int L, cudaStream_t s);
 
 void sinusoid_freqs_host(int dim, float* hf /*[dim / 2]*/);
 void launch_sinusoid(float* out, const float* freq_dev, int T, int dim, cudaStream_t s);

@@ -855,47 +855,26 @@ void launch_softattn(const T* qkv, int ld, T* out, int ld_out, int n_scenes, int
   k_softattn<T><<<n_scenes, 128, smem, s>>>(qkv, ld, out, ld_out, n_scenes, n_obj);
 }
 
-// cross linear attention -- text side, once per sampling call: ctx[scene][h][d][e] (fp32)
-__global__ void __launch_bounds__(128) k_xattn_prepare(const float* __restrict__ kv, int ld_kv,
-                                                       float* __restrict__ ctx, int n_scenes, int L) {
-  extern __shared__ float sm[];
+// cross linear attention -- text side: ctx[scene][h][d][e] (fp32) from the scene's L rows of k | v (storage type T).
+// Once per sampling call (ds_set_context_cross) and once per training step.  One CTA per scene, one warp per head;
+// the tokens are streamed in chunks (common.cuh), so every L the API accepts (<= 512) launches.
+template <typename T>
+__global__ void __launch_bounds__(128) k_xattn_prepare(const T* __restrict__ kv, int ld_kv, float* __restrict__ ctx, int L) {
+  __shared__ float sm[4][2][XATTN_CHUNK][33];
   const int lane = threadIdx.x & 31, h = threadIdx.x >> 5;
   const int scene = blockIdx.x;
-  float* ks = sm + h * 2 * L * 32;
-  float* vs = ks + L * 32;
-  const int64_t row0 = (int64_t)scene * L;
-  float kmax = -INFINITY;
-  for (int l = 0; l < L; ++l) {
-    const float* p = kv + (row0 + l) * ld_kv + h * 32 + lane;
-    float k = p[0];
-    ks[l * 32 + lane] = k;
-    vs[l * 32 + lane] = p[128];
-    kmax = fmaxf(kmax, k);
-  }
-  float ksum = 0.f;
-  for (int l = 0; l < L; ++l) {
-    float e = expf(ks[l * 32 + lane] - kmax);
-    ks[l * 32 + lane] = e;
-    ksum += e;
-  }
-  const float kinv = 1.0f / ksum;
-  for (int l = 0; l < L; ++l) ks[l * 32 + lane] *= kinv;
-  __syncwarp();
-  float acc[32];
-#pragma unroll
-  for (int d = 0; d < 32; ++d) acc[d] = 0.f;
-  for (int l = 0; l < L; ++l) {
-    float v = vs[l * 32 + lane];
-#pragma unroll
-    for (int d = 0; d < 32; ++d) acc[d] += ks[l * 32 + d] * v;
-  }
+  const T* kvs = kv + (int64_t)scene * L * ld_kv;
+  float kmax, kinv;
+  xattn_k_stats(kvs, ld_kv, L, h, lane, kmax, kinv);
+  float acc[32];      // lane = e: acc[d] = ctx[d][e]
+  xattn_context<T, false>(kvs, ld_kv, L, h, lane, kmax, kinv, sm[h][0], sm[h][1], acc);
   float* o = ctx + ((int64_t)scene * 4 + h) * 1024;
 #pragma unroll
   for (int d = 0; d < 32; ++d) o[d * 32 + lane] = acc[d];
 }
-void launch_xattn_prepare(const float* kv, int ld_kv, float* ctx, int n_scenes, int L, cudaStream_t s) {
-  size_t smem = size_t(4) * 2 * L * 32 * sizeof(float);
-  k_xattn_prepare<<<n_scenes, 128, smem, s>>>(kv, ld_kv, ctx, n_scenes, L);
+template <typename T>
+void launch_xattn_prepare(const T* kv, int ld_kv, float* ctx, int n_scenes, int L, cudaStream_t s) {
+  if (n_scenes > 0) k_xattn_prepare<T><<<n_scenes, 128, 0, s>>>(kv, ld_kv, ctx, L);
 }
 
 template <typename T>
@@ -1334,7 +1313,6 @@ void init_pointwise_attrs() {
   cudaFuncSetAttribute(k_linattn<bf16, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
   cudaFuncSetAttribute(k_softattn<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
   cudaFuncSetAttribute(k_softattn<bf16>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
-  cudaFuncSetAttribute(k_xattn_prepare, cudaFuncAttributeMaxDynamicSharedMemorySize, lim);
 }
 
 // ---- explicit instantiations ----
@@ -1347,6 +1325,7 @@ void init_pointwise_attrs() {
   template void launch_linattn<T>(const T*, int, T*, int, int, int, cudaStream_t);                                \
   template void launch_softattn<T>(const T*, int, T*, int, int, int, cudaStream_t);                               \
   template void launch_xattn_apply<T>(const T*, int, const float*, T*, int, int, int, cudaStream_t);              \
+  template void launch_xattn_prepare<T>(const T*, int, float*, int, int, cudaStream_t);                           \
   template void launch_step_update<T>(const StepCoef*, StepState*, float*, const T*, int, const float*, int, int, \
                                       int, int, cudaStream_t);                                                    \
   template void launch_p_sample<T>(const float*, const T*, int, const int*, const float*, float*, const float*,   \

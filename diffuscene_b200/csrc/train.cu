@@ -8,6 +8,8 @@
 // the host.  The training step program is the plan of plan.cpp in train mode (one op per reference layer); its
 // adjoint is executed op by op in reverse (kernels: backward.cu).  The time-embedding MLP and the 19 + 9 FiLM
 // projections run per sample here (fp32), not from the hoisted tables of the sampling path: their weights are trained.
+// Likewise the text side of the cross-attention layers (to_kv projection, softmax over the tokens, k^T v context) is
+// computed every step from the flat parameters and differentiated down to d(to_kv.weight) and d(context_cross).
 #include "engine_internal.h"
 
 namespace ds {
@@ -32,6 +34,9 @@ void launch_ln_bwd(const T* x, int ldx, const T* dy, int ldy, T* dx, int lddx, i
                    int res_accumulate, const float* g, float* dg, int M, int C, cudaStream_t s);
 template <typename T> void launch_linattn_bwd(const T* qkv, int ld, const T* dout, int ldo, T* dqkv, int lddq, int n_scenes, int N, cudaStream_t s);
 template <typename T> void launch_softattn_bwd(const T* qkv, int ld, const T* dout, int ldo, T* dqkv, int lddq, int n_scenes, int N, cudaStream_t s);
+template <typename T>
+void launch_xattn_bwd(const T* q, int ldq, const T* dout, int ldo, const T* kv, int ld_kv, T* dq, int lddq, int dq_accumulate,
+                      T* dkv, int ld_dkv, int n_scenes, int n_obj, int L, cudaStream_t s);
 template <typename T>
 void launch_p_losses_bwd(const float* x0, const float* noise, const float* x_t, const T* out, int ld, const int64_t* t,
                          const float* sqrt_ac, const float* sqrt_1mac, const float* sqrt_recip_ac,
@@ -159,6 +164,20 @@ struct TrainState {
   // flat buffer from its END towards its start: parameters are laid out in forward order)
   std::vector<int64_t> bucket_bounds;
   std::vector<cudaEvent_t> bucket_events;
+  // text condition (ds_train_set_context_cross; the pointers are borrowed).  The to_kv projections of all cross-attention
+  // layers run as ONE GEMM: kv [B*L, NKV] = context_cross [B*L, TD] x kvw^T, kvw = the layers' to_kv weights stacked
+  // [NKV = layers * 256, TD] in storage dtype.  bf16 with the tcgen05 backend (`text_tc`): the forward, d(to_kv.weight)
+  // (split-K on the transposed copies trKV = dkv_l^T, crossT) and d(context_cross) = dkv x kvw (kvwT: K-major copy)
+  // run on the tensor cores
+  const float* cross = nullptr;
+  float* dcross = nullptr;
+  int cross_batch = 0, cross_L = 0;
+  bool text_tc = false;
+  int x_rows_cap = 0, x_rows_pad = 0, x_scenes_cap = 0;
+  void *kvw = nullptr, *kv = nullptr, *dkv = nullptr;
+  float* xctx = nullptr;                 // [layers][B][4][32][32] text context of every layer
+  ds::bf16 *kvwT = nullptr, *cross_bf = nullptr, *crossT = nullptr, *trKV = nullptr, *dcross_bf = nullptr;
+  TcGemmPlan *tc_kv = nullptr, *tc_kvdw = nullptr, *tc_dcross = nullptr;
   cudaEvent_t ev[7] = {nullptr};      // phase boundaries of the last step (ds_train_phase_ms)
   bool ev_valid = false;
 };
@@ -184,6 +203,10 @@ void train_state_destroy(TrainState* t) {
   if (t->tc_dst) tc_plan_destroy(t->tc_dst);
   for (ds::bf16* p : {t->st_bf, t->film_bf, t->dfilm_bf, t->dst_bf, t->wall_bf, t->wallT_bf, t->trF, t->stT}) cudaFree(p);
   cudaFree(t->ball);
+  for (void* p : {t->kvw, t->kv, t->dkv, (void*)t->xctx, (void*)t->kvwT, (void*)t->cross_bf, (void*)t->crossT, (void*)t->trKV,
+                  (void*)t->dcross_bf})
+    cudaFree(p);
+  for (auto* p : {t->tc_kv, t->tc_kvdw, t->tc_dcross}) if (p) tc_plan_destroy(p);
   delete t;
 }
 
@@ -191,8 +214,6 @@ static int train_round_up(int a, int b) { return (a + b - 1) / b * b; }
 
 static int train_init(ds_handle* h) {
   if (h->train) return 0;
-  if (h->cfg.text_condition)
-    return fail(DS_ERR_INVALID, "native training supports the unconditional / arrangement networks (no cross-attention backward)");
   TrainState* t = new TrainState();
   ds_config cfg = h->cfg;
   cfg.train = 1;
@@ -247,8 +268,87 @@ static int train_init(ds_handle* h) {
   t->v_total = vt;
   CK(cudaMalloc(&t->varena, vt * 4));
   CK(cudaMalloc(&t->dvarena, vt * 4));
+  if (h->cfg.text_condition) {
+    const int TD = h->cfg.text_dim, NKV = int(P.xattn_layers.size()) * 256;
+    t->text_tc = t->use_tc && TD % 128 == 0;      // tcgen05 shape rules: K % 64 and N % 128 (TD is both)
+    CK(cudaMalloc(&t->kvw, (size_t)NKV * TD * t->esz));
+    if (t->text_tc) CK(cudaMalloc(&t->kvwT, (size_t)TD * NKV * 2));
+  }
   h->train = t;
   return 0;
+}
+
+// text buffers and plans for B scenes of L tokens; grown (never shrunk) like train_capacity's, since L follows the
+// longest description of each batch
+static int train_text_capacity(ds_handle* h, int B, int L) {
+  TrainState* t = h->train;
+  const int nl = int(t->plan.xattn_layers.size()), TD = h->cfg.text_dim, NKV = nl * 256;
+  if (B > t->x_scenes_cap) {
+    cudaFree(t->xctx);
+    t->xctx = nullptr;
+    CK(cudaMalloc(&t->xctx, (size_t)nl * B * 4096 * 4));
+    t->x_scenes_cap = B;
+  }
+  const int rows = B * L;
+  if (rows <= t->x_rows_cap) return 0;
+  for (void* p : {t->kv, t->dkv, (void*)t->cross_bf, (void*)t->crossT, (void*)t->trKV, (void*)t->dcross_bf}) cudaFree(p);
+  t->kv = t->dkv = nullptr;
+  t->cross_bf = t->crossT = t->trKV = t->dcross_bf = nullptr;
+  for (TcGemmPlan** p : {&t->tc_kv, &t->tc_kvdw, &t->tc_dcross}) {
+    if (*p) tc_plan_destroy(*p);
+    *p = nullptr;
+  }
+  t->x_rows_cap = t->x_rows_pad = 0;
+  const int rp = train_round_up(rows, 128);
+  auto alloc0 = [&](void** p, size_t bytes) { cudaError_t e = cudaMalloc(p, bytes); if (e == cudaSuccess) e = cudaMemset(*p, 0, bytes); return e; };
+  CK(alloc0(&t->kv, (size_t)rp * NKV * t->esz));
+  CK(alloc0(&t->dkv, (size_t)rp * NKV * t->esz));
+  if (t->bf16) {
+    CK(alloc0((void**)&t->cross_bf, (size_t)rp * TD * 2));
+    CK(alloc0((void**)&t->dcross_bf, (size_t)rp * TD * 2));
+  }
+  if (t->text_tc) {
+    CK(alloc0((void**)&t->crossT, (size_t)TD * rp * 2));
+    CK(alloc0((void**)&t->trKV, (size_t)256 * rp * 2));
+    char err[256] = "";
+    GemmArgs g;
+    memset(&g, 0, sizeof g);
+    g.no_pair = 1;      // training GEMMs stay single-CTA (kernels.cuh)
+    g.a0 = t->cross_bf; g.lda0 = TD; g.k0 = TD;
+    g.w = t->kvw; g.ldw = TD;
+    g.d = t->kv; g.ldd = NKV;
+    g.M = rp; g.N = NKV;
+    if (!(t->tc_kv = tc_plan_create(g, rp, err, sizeof err))) return fail(DS_ERR_CUDA, "train: to_kv plan failed: %s", err);
+    // d(to_kv.weight) of one layer = dkv_l^T x context_cross: A = trKV [256, rp], "weights" = crossT [TD, rp]
+    memset(&g, 0, sizeof g);
+    g.no_pair = 1;
+    g.a0 = t->trKV; g.lda0 = rp; g.k0 = rp;
+    g.w = t->crossT; g.ldw = rp;
+    g.d = t->trKV; g.ldd = 8;             // placeholder (bf16 output unused in atomic mode)
+    g.M = 256; g.N = TD;
+    if (!(t->tc_kvdw = tc_plan_create(g, 256, err, sizeof err)))
+      return fail(DS_ERR_CUDA, "train: to_kv weight-gradient plan failed: %s", err);
+    // d(context_cross) = dkv [rows, NKV] x kvw [NKV, TD]: "weights" = kvwT [TD, NKV]
+    memset(&g, 0, sizeof g);
+    g.no_pair = 1;
+    g.a0 = t->dkv; g.lda0 = NKV; g.k0 = NKV;
+    g.w = t->kvwT; g.ldw = NKV;
+    g.d = t->dcross_bf; g.ldd = TD;
+    g.M = rp; g.N = TD;
+    if (!(t->tc_dcross = tc_plan_create(g, rp, err, sizeof err)))
+      return fail(DS_ERR_CUDA, "train: d(context_cross) plan failed: %s", err);
+  }
+  t->x_rows_cap = rows;
+  t->x_rows_pad = rp;
+  return 0;
+}
+
+// split-K factor of a dW GEMM with `tiles` output tiles over `kblocks` 64-deep k-blocks: one wave of CTAs, every split
+// owning at least one k-block (the kernel derives its k-blocks per split the same way)
+static int train_ksplit(int tiles, int kblocks) {
+  int ksplit = std::max(1, std::min(148 / std::max(1, tiles), kblocks));
+  const int kb_per = (kblocks + ksplit - 1) / ksplit;
+  return (kblocks + kb_per - 1) / kb_per;
 }
 
 static int train_capacity(ds_handle* h, int n_scenes, int ctx_rows) {
@@ -466,6 +566,11 @@ static int train_step_t(ds_handle* h, const float* flat, const float* x0, const 
                            r.K, r.ws ? 1 : 0,
                            t->use_tc ? (T*)(t->wtarena + t->w_off[i]) + (size_t)pc.col_off * r.N + pc.row_off : nullptr, r.N, s);
   }
+  const bool text = c.text_condition != 0;
+  const int TD = c.text_dim, NKV = int(P.xattn_layers.size()) * 256, XL = t->cross_L, XR = B * XL;
+  for (size_t l = 0; text && l < P.xattn_layers.size(); ++l)
+    launch_pack_piece<T>(F(P.xattn_layers[l] + ".fn.fn.to_kv.weight"), 256, TD, (T*)t->kvw + l * 256 * TD, TD, 0,
+                         t->text_tc ? (T*)(void*)t->kvwT + l * 256 : nullptr, NKV, s);
   CK(cudaMemsetAsync(t->varena, 0, t->v_total * 4, s));
   for (size_t i = 0; i < P.vecs.size(); ++i)
     for (const VPiece& pc : P.vecs[i].pieces)
@@ -520,6 +625,26 @@ static int train_step_t(ds_handle* h, const float* flat, const float* x0, const 
   for (int i = 0; i < ncb; ++i)
     f32gemm(t->ctx_act, E, E, F(P.ctx_blocks[i] + ".mlp.1.weight"), F(P.ctx_blocks[i] + ".mlp.1.bias"),
             t->ctx_film + (size_t)i * 2 * C, ncb * 2 * C, 2 * C, ctx_rows);
+  if (text) {
+    // k | v of every cross-attention layer in one GEMM, then each layer's text context [B, 4, 32, 32]
+    if (t->bf16) {
+      k_f32_to_bf16<<<((int64_t)XR * TD + 255) / 256, 256, 0, s>>>(t->cross, TD, t->cross_bf, TD, XR, TD);
+      h->launches++;
+    }
+    if (t->text_tc) {
+      int e = launch_gemm_tc(t->tc_kv, XR, s);
+      if (e) return fail(DS_ERR_CUDA, "train: to_kv GEMM failed: %s", cudaGetErrorString((cudaError_t)e));
+    } else {
+      memset(&g, 0, sizeof g);
+      g.a0 = t->bf16 ? (const void*)t->cross_bf : (const void*)t->cross; g.lda0 = TD; g.k0 = TD;
+      g.w = t->kvw; g.ldw = TD; g.d = t->kv; g.ldd = NKV; g.M = XR; g.N = NKV; g.act = ACT_NONE;
+      if constexpr (sizeof(T) == 4) launch_gemm_f32(g, s);
+      else launch_gemm_simt<T>(g, true, s);
+    }
+    for (size_t l = 0; l < P.xattn_layers.size(); ++l)
+      launch_xattn_prepare<T>((const T*)t->kv + l * 256, NKV, t->xctx + l * B * 4096, B, XL, s);
+    h->launches += 1 + int(P.xattn_layers.size());
+  }
 
   auto film_of = [&](const Op& o) {
     FilmRef f;
@@ -573,6 +698,10 @@ static int train_step_t(ds_handle* h, const float* flat, const float* x0, const 
         break;
       case OP_ATTN:
         launch_softattn<T>(ptr(o.in0.buf, 0), ld(o.in0.buf), ptr(o.out, 0), ld(o.out), B, n_obj, s);
+        break;
+      case OP_XATTN:
+        launch_xattn_apply<T>(ptr(o.in0.buf, 0), ld(o.in0.buf), t->xctx + (size_t)o.xlayer * B * 4096, ptr(o.out, 0), ld(o.out),
+                              B, n_obj, s);
         break;
       default:
         return fail(DS_ERR_STATE, "op kind %d has no training path", o.kind);
@@ -663,7 +792,7 @@ static int train_step_t(ds_handle* h, const float* flat, const float* x0, const 
     return 0;
   };
   bool dst_started = false, dctx_started = false;
-  bool stT_ready = false;
+  bool stT_ready = false, crossT_ready = false;
   auto time_block_bwd = [&](int i) {      // FiLM projection of time block i: dW, db, and its share of d(SiLU(temb))
     const float* df = t->dfilm + (size_t)i * 2 * C;
     if (film_tc) {
@@ -792,6 +921,29 @@ static int train_step_t(ds_handle* h, const float* flat, const float* x0, const 
         launch_softattn_bwd<T>(ptr(o.in0.buf, 0), ld(o.in0.buf), gptr(o.out, 0), ld(o.out), gptr(o.in0.buf, 0), ld(o.in0.buf), B,
                                n_obj, s);
         break;
+      case OP_XATTN: {
+        // dq and this layer's d(k | v) [B*L, 256], then d(to_kv.weight) = dkv_l^T x context_cross (final here)
+        const int acc = first_write(o.in0.buf, 0);
+        T* dkv_l = (T*)t->dkv + (size_t)o.xlayer * 256;
+        launch_xattn_bwd<T>(ptr(o.in0.buf, 0), ld(o.in0.buf), gptr(o.out, 0), ld(o.out), (const T*)t->kv + (size_t)o.xlayer * 256,
+                            NKV, gptr(o.in0.buf, 0), ld(o.in0.buf), acc, dkv_l, NKV, B, n_obj, XL, s);
+        const std::string wn = P.xattn_layers[o.xlayer] + ".fn.fn.to_kv.weight";
+        if (t->text_tc) {
+          if (!crossT_ready) {
+            launch_transpose_pad<bf16>(t->cross_bf, TD, t->crossT, t->x_rows_pad, XR, t->x_rows_pad, TD, nullptr, s);
+            crossT_ready = true;
+          }
+          launch_transpose_pad<bf16>((const bf16*)(void*)dkv_l, NKV, t->trKV, t->x_rows_pad, XR, t->x_rows_pad, 256, nullptr, s);
+          tc_plan_set_atomic_out(t->tc_kvdw, G(wn), TD, train_ksplit(tc_plan_tiles(t->tc_kvdw, 256), t->x_rows_pad / 64));
+          int e = launch_gemm_tc(t->tc_kvdw, 256, s);
+          if (e) return fail(DS_ERR_CUDA, "train: to_kv dW GEMM failed: %s", cudaGetErrorString((cudaError_t)e));
+        } else {
+          launch_gemm_tn<T, T>(dkv_l, NKV, t->bf16 ? (const T*)(const void*)t->cross_bf : (const T*)(const void*)t->cross, TD,
+                               G(wn), TD, XR, 256, TD, s);
+        }
+        pending[wn] = false;
+        break;
+      }
       default:
         return fail(DS_ERR_STATE, "op kind %d has no backward", o.kind);
     }
@@ -816,6 +968,17 @@ static int train_step_t(ds_handle* h, const float* flat, const float* x0, const 
   for (const char* n : {"time_mlp.1.weight", "time_mlp.1.bias", "time_mlp.3.weight", "time_mlp.3.bias"}) pending[n] = false;
   if (dcontext)
     k_mul_actgrad<<<((int64_t)ctx_rows * E + 255) / 256, 256, 0, s>>>(t->dctx_act, context, dcontext, (int64_t)ctx_rows * E, ACT_SILU);
+  if (text && t->dcross) {      // d(context_cross) = sum over layers of dkv_l x W_kv,l: one GEMM with K = NKV
+    if (t->text_tc) {
+      int e = launch_gemm_tc(t->tc_dcross, XR, s);
+      if (e) return fail(DS_ERR_CUDA, "train: d(context_cross) GEMM failed: %s", cudaGetErrorString((cudaError_t)e));
+    } else {
+      launch_gemm_nn<T, T, T>((const T*)t->dkv, NKV, (const T*)t->kvw, TD, t->bf16 ? (T*)(void*)t->dcross_bf : (T*)(void*)t->dcross,
+                              TD, XR, TD, NKV, 0, s);
+    }
+    if (t->bf16) k_bf16_to_f32<<<((int64_t)XR * TD + 255) / 256, 256, 0, s>>>(t->dcross_bf, TD, t->dcross, TD, XR, TD);
+    h->launches++;
+  }
   cudaEventRecord(t->ev[5], s);
   // ---- 6. every named gradient is final: release the remaining buckets
   for (auto& kv : pending)
@@ -850,6 +1013,12 @@ extern "C" int ds_train_step(ds_handle* h, const float* flat_params_dev, const f
   if (rc) return rc;
   const int ctx_rows = ctx_shared ? h->cfg.num_objects : ctx_batch * h->cfg.num_objects;
   if ((rc = train_capacity(h, batch, ctx_rows))) return rc;
+  if (h->cfg.text_condition) {
+    if (!h->train->cross) return fail(DS_ERR_STATE, "text network: ds_train_set_context_cross() has not been called");
+    if (h->train->cross_batch != batch)
+      return fail(DS_ERR_STATE, "context_cross was set for batch %d, call uses batch %d", h->train->cross_batch, batch);
+    if ((rc = train_text_capacity(h, batch, h->train->cross_L))) return rc;
+  }
   cudaStream_t s = (cudaStream_t)stream;
   if (h->train->bf16)
     return train_step_t<bf16>(h, flat_params_dev, x0_dev, t_dev, noise_dev, context_dev, ctx_batch, ctx_shared, loss_separate,
@@ -869,6 +1038,29 @@ extern "C" int ds_train_set_buckets(ds_handle* h, const int64_t* bounds, int32_t
   for (int i = 0; i < n_buckets; ++i) t->bucket_events.push_back((cudaEvent_t)events[i]);
   if (n_buckets > 0 && (t->bucket_bounds.front() != 0 || t->bucket_bounds.back() != t->flat_n))
     return fail(DS_ERR_INVALID, "bucket bounds must run from 0 to ds_train_param_count()");
+  return 0;
+}
+
+extern "C" int ds_train_set_context_cross(ds_handle* h, const float* cross_dev, int32_t batch, int32_t L, float* dcross_dev) {
+  if (!h) return fail(DS_ERR_INVALID, "null handle");
+  if (!h->cfg.text_condition) return fail(DS_ERR_INVALID, "configuration has no text condition");
+  if (!cross_dev) {
+    if (h->train) {
+      h->train->cross = nullptr;
+      h->train->dcross = nullptr;
+      h->train->cross_batch = h->train->cross_L = 0;
+    }
+    return 0;
+  }
+  if (batch <= 0 || L <= 0 || L > 512) return fail(DS_ERR_INVALID, "bad context_cross shape (batch %d, L %d)", batch, L);
+  CK(cudaSetDevice(h->cfg.device));
+  int rc = train_init(h);
+  if (rc) return rc;
+  TrainState* t = h->train;
+  t->cross = cross_dev;
+  t->dcross = dcross_dev;
+  t->cross_batch = batch;
+  t->cross_L = L;
   return 0;
 }
 

@@ -239,9 +239,13 @@ class DenoiserEngine:
     def train_step(self, flat_params: torch.Tensor, x0: torch.Tensor, t: torch.Tensor, noise: torch.Tensor,
                    context: torch.Tensor, shared: bool, loss_separate: bool, loss_iou: bool,
                    bounds: Optional[Sequence[float]] = None, flat_grads: Optional[torch.Tensor] = None,
-                   want_dcontext: bool = True, grad_scale: float = 1.0):
+                   want_dcontext: bool = True, grad_scale: float = 1.0,
+                   context_cross: Optional[torch.Tensor] = None):
         """Forward of p_losses + the native backward pass: (losses [B], loss dict, d(context) or None).
-        Gradients of every denoiser parameter land in `flat_grads` (flat_layout order)."""
+        Gradients of every denoiser parameter land in `flat_grads` (flat_layout order).
+
+        Text-conditioned networks pass `context_cross` [B, L, text_dim] (the input of every cross-attention to_kv);
+        the result then has a fourth entry, d(context_cross) (None without flat_grads)."""
         assert flat_params.is_cuda and flat_params.dtype == torch.float32 and flat_params.is_contiguous()
         x0, t, noise = x0.contiguous(), t.to(self.device).contiguous(), noise.contiguous()
         ctx = context.detach().to(self.device, torch.float32).contiguous()
@@ -250,11 +254,22 @@ class DenoiserEngine:
         ld = torch.empty(9, device=self.device, dtype=torch.float32)
         dctx = torch.empty_like(ctx) if (want_dcontext and flat_grads is not None) else None
         barr = None if bounds is None else (C.c_float * 12)(*[float(v) for v in bounds])
-        capi.check(self.lib.ds_train_step(self.h, _ptr(flat_params), _ptr(x0), _ptr(t), _ptr(noise), _ptr(ctx),
-                                          0 if shared else B, int(bool(shared)), int(loss_separate), int(loss_iou), barr,
-                                          float(grad_scale), _ptr(losses), _ptr(ld), _ptr(flat_grads), _ptr(dctx), B,
-                                          self._stream()))
-        return losses, {k: ld[i] for i, k in enumerate(LOSS_KEYS)}, dctx
+        cross = dcross = None
+        if context_cross is not None:
+            cross = context_cross.detach().to(self.device, torch.float32).contiguous()
+            dcross = torch.empty_like(cross) if flat_grads is not None else None
+            capi.check(self.lib.ds_train_set_context_cross(self.h, _ptr(cross), cross.shape[0], cross.shape[1],
+                                                           _ptr(dcross)))
+        try:
+            capi.check(self.lib.ds_train_step(self.h, _ptr(flat_params), _ptr(x0), _ptr(t), _ptr(noise), _ptr(ctx),
+                                              0 if shared else B, int(bool(shared)), int(loss_separate), int(loss_iou),
+                                              barr, float(grad_scale), _ptr(losses), _ptr(ld), _ptr(flat_grads),
+                                              _ptr(dctx), B, self._stream()))
+        finally:
+            if cross is not None:      # the handle only borrows the pointers: never leave them behind
+                capi.check(self.lib.ds_train_set_context_cross(self.h, None, 0, 0, None))
+        out = (losses, {k: ld[i] for i, k in enumerate(LOSS_KEYS)}, dctx)
+        return out + (dcross,) if context_cross is not None else out
 
     def train_set_buckets(self, bounds: Sequence[int], events: Sequence["torch.cuda.Event"]):
         """Gradient buckets for the overlapped all-reduce (see ds_train_set_buckets); `events` are torch.cuda.Event

@@ -7,9 +7,9 @@ Same constructor arguments, same public methods (`get_loss`, `sample`, `generate
 `fc_*`), so reference checkpoints load unchanged.  Parameters are fp32 `nn.Parameter`s (the master copy the
 optimizer updates); the engine keeps a packed copy that is refreshed lazily when the parameters change.
 
-Sampling, validation loss and every diffusion step run in the CUDA library.  The training backward pass is
-torch autograd over `functional.DenoiserFn` on the same parameters (see DESIGN.md: native backward is future
-work).  Differences from the reference that are deliberate: the per-call `print`s are gone, `sample()` honours
+Sampling, validation loss, every diffusion step and the training step (forward and backward pass of the denoiser,
+`ds_train_step`) run in the CUDA library; `native_backward = False` differentiates `functional.DenoiserFn` with
+torch autograd instead (the reference path the tests compare against).  Differences from the reference that are deliberate: the per-call `print`s are gone, `sample()` honours
 `ddim=True` (the reference ignores it and its DDIM loop is dead code), and emptiness is decided per scene when
 batch_size > 1 via `delete_empty_batched` (the reference looks at batch row 0 only).  Like the reference
 (`sample()` dispatches on input_boxes / partial_boxes first, :293-299), `complete_scene` / `arrange_scene` accept
@@ -48,22 +48,23 @@ def _register(root: nn.Module, dotted: str, param: nn.Parameter):
 
 class _NativeTrainLoss(torch.autograd.Function):
     """p_losses(...).mean() with the forward AND the backward pass of the denoiser in the CUDA library (ds_train_step).
-    The only differentiable input is the conditioning tensor (its gradient flows on into positional_embedding / the
-    condition MLPs through ordinary autograd); the denoiser parameters receive their gradients as views of the
-    model's flat gradient buffer when backward() runs."""
+    The differentiable inputs are the conditioning tensor and, for text networks, `context_cross` (their gradients
+    flow on into positional_embedding / the condition MLPs / fc_text_f through ordinary autograd); the denoiser
+    parameters receive their gradients as views of the model's flat gradient buffer when backward() runs."""
 
     @staticmethod
-    def forward(ctx, cond, model, x0, t, noise, shared):
-        losses, ld, dcond = model._native_fwd_bwd(x0, t, noise, cond, shared)
-        ctx.model, ctx.dcond = model, dcond
+    def forward(ctx, cond, cross, model, x0, t, noise, shared):
+        losses, ld, dcond, dcross = model._native_fwd_bwd(x0, t, noise, cond, shared, cross)
+        ctx.model, ctx.dcond, ctx.dcross = model, dcond, dcross
         model._last_loss_dict = ld
         return losses.mean()
 
     @staticmethod
     def backward(ctx, g):
         ctx.model._assign_native_grads(g)
-        d = ctx.dcond
-        return (None if d is None else d * g), None, None, None, None, None
+        d, dx = ctx.dcond, ctx.dcross
+        dx = dx * g if (dx is not None and ctx.needs_input_grad[1]) else None
+        return (None if d is None else d * g), dx, None, None, None, None, None
 
 
 class DiffusionSceneLayout_DDPM(nn.Module):
@@ -219,7 +220,7 @@ class DiffusionSceneLayout_DDPM(nn.Module):
 
     # ---- native training: flat parameter / gradient buffers ---------------------------------------
     def native_training_supported(self) -> bool:
-        return (not self.text_condition) and self.sample_num_points <= 32 and self._device().type == "cuda"
+        return self.sample_num_points <= 32 and self._device().type == "cuda"
 
     def _ensure_flat(self):
         """All denoiser parameters as views into ONE flat fp32 device buffer (ds_expected_weight order), gradients
@@ -246,20 +247,22 @@ class DiffusionSceneLayout_DDPM(nn.Module):
         self._overlap = None
         return eng
 
-    def _native_fwd_bwd(self, x0, t, noise, cond, shared):
+    def _native_fwd_bwd(self, x0, t, noise, cond, shared, cross=None):
         eng = self._ensure_flat()
         world = torch.distributed.get_world_size() if (torch.distributed.is_available() and torch.distributed.is_initialized()) else 1
         if world > 1 and self._overlap is None:
             from ..parallel import GradOverlap
             self._overlap = GradOverlap(eng, self._flat_grads)
-        losses, ld, dcond = eng.train_step(self._flat, x0, t, noise, cond, shared, self.loss_separate, self.loss_iou,
-                                           self.bounds, flat_grads=self._flat_grads, grad_scale=1.0 / world)
+        res = eng.train_step(self._flat, x0, t, noise, cond, shared, self.loss_separate, self.loss_iou, self.bounds,
+                             flat_grads=self._flat_grads, grad_scale=1.0 / world, context_cross=cross)
+        losses, ld, dcond = res[:3]
+        dcross = res[3] if cross is not None else None
         if world > 1:
             # the kernels of the backward pass are only ENQUEUED at this point: the bucket all-reduces go to a side
             # stream, each gated by the event the engine records when that bucket's gradients are final
             self._overlap.launch()
         self._native_grads_ready = False
-        return losses, ld, dcond
+        return losses, ld, dcond, dcross
 
     def _assign_native_grads(self, g):
         """Called from the autograd node of the native loss: expose the flat gradient buffer as the .grad of every
@@ -372,7 +375,7 @@ class DiffusionSceneLayout_DDPM(nn.Module):
         if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
             if self.native_backward and self.native_training_supported():
                 c = cond if cond.requires_grad else cond.detach().requires_grad_(True)
-                loss = _NativeTrainLoss.apply(c, self, target, t, noise, shared)
+                loss = _NativeTrainLoss.apply(c, cross, self, target, t, noise, shared)
                 ld = self._last_loss_dict
                 if self.room_arrange_condition:
                     ld = {k: ld[k] for k in ("loss.trans", "loss.angle")}

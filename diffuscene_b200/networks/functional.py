@@ -1,9 +1,10 @@
-"""Differentiable (torch autograd) forward of the denoiser used ONLY for training on the GPU.
+"""Differentiable (torch autograd) forward of the denoiser: the reference training path.
 
-The native CUDA engine implements the forward of every op (sampling, validation loss); backward kernels are
-not written yet, so `train_on_batch` differentiates this functional form with torch autograd on the same
-parameters (a library path, stated as such in DESIGN.md).  Semantics: reference
-scene_synthesis/networks/denoise_net.py:507-593 in token-major layout.
+`train_on_batch` runs the native CUDA training step (ds_train_step: forward and hand-written backward pass) for
+every network the library builds, text-conditioned ones included.  This functional form is what a model with
+`native_backward = False` differentiates with torch autograd instead, on the same parameters; the tests compare
+the native step against it.  Semantics: reference scene_synthesis/networks/denoise_net.py:507-593 in
+token-major layout.
 """
 from __future__ import annotations
 

@@ -187,13 +187,22 @@ DS_API int ds_p_losses(ds_handle* h, const float* x0_dev, const int64_t* t_dev, 
  * data-parallel mean after a sum all-reduce.  context [ctx_shared ? N : B*N, cond_dim] is the conditioning input of
  * Unet1D.forward; dcontext_dev (optional, same shape) receives its gradient (it continues into
  * positional_embedding / the condition MLPs on the caller's side).  flat_grads_dev == NULL: forward + loss only.
- * Uses the handle's schedule (ds_set_schedule) and precision; networks with text cross-attention are not supported. */
+ * Uses the handle's schedule (ds_set_schedule) and precision.  Networks with text cross-attention (text_condition)
+ * need ds_train_set_context_cross() for the same batch first: their to_kv projections run from flat_params_dev on
+ * every step, and d(to_kv.weight) lands in flat_grads_dev like every other gradient. */
 DS_API int64_t ds_train_param_count(ds_handle* h);
 DS_API int ds_train_step(ds_handle* h, const float* flat_params_dev, const float* x0_dev, const int64_t* t_dev,
                          const float* noise_dev, const float* context_dev, int32_t ctx_batch, int32_t ctx_shared,
                          int32_t loss_separate, int32_t loss_iou, const float* bounds_host, float grad_scale,
                          float* losses_dev, float* loss_dict_dev, float* flat_grads_dev, float* dcontext_dev,
                          int32_t batch, void* stream);
+/* Text condition of the following ds_train_step calls: context_cross [batch, L, text_dim] fp32 device (the input of
+ * every LinearAttentionCross's to_kv, denoise_net.py:261-297), 1 <= L <= 512.  dcross_dev (optional, same shape)
+ * receives d(loss)/d(context_cross) on every ds_train_step that computes gradients; it continues into fc_text_f on
+ * the caller's side.  Pointers are borrowed until the next call; cross_dev == NULL clears.  A ds_train_step on a text
+ * network without it, or with a different batch, fails with DS_ERR_STATE; a network without text condition gives
+ * DS_ERR_INVALID. */
+DS_API int ds_train_set_context_cross(ds_handle* h, const float* cross_dev, int32_t batch, int32_t L, float* dcross_dev);
 /* Overlap of the data-parallel gradient all-reduce with the backward pass: bucket k is the flat range
  * [bounds[k], bounds[k + 1]) (bounds[0] = 0, bounds[n] = ds_train_param_count()); ds_train_step records events[k] (a
  * cudaEvent_t owned by the caller) on its stream as soon as every gradient inside the bucket is final -- the backward
